@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark: Msamples/s of the path-tracing hot path on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c1|c2|c3] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c1|c2|c3] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one run_view of the whole frame (all spp). With N > 1 the samples are sharded over the
@@ -279,9 +279,38 @@ class Ctx:
             self.torch.distributed.destroy_process_group()
 
 
-def render_workload(ctx, name, steps, warmup, estimator=0, headline=False, clocks=False, prebuilt=None):
+DUMP_BYTES = 64 * 10 ** 6     # --dump-outputs: at most this many bytes of .npy files per run
+DUMP_SEED = 0
+
+
+def dump_sample_index(n, bytes_per_item):
+    """Sorted indices of a fixed, seeded sample of n items that fits DUMP_BYTES with room for the .npy headers (all of
+    them when they fit): the same arguments give the same indices on every run and every build."""
+    import numpy as np
+    k = min(n, (DUMP_BYTES - 4096) // bytes_per_item)
+    if k == n:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=k, replace=False))
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes {name: array} as out_dir/<name>.npy (float32 / float64 only, DUMP_BYTES in all)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, a)
+        total += os.path.getsize(path)
+    assert total <= DUMP_BYTES, total
+
+
+def render_workload(ctx, name, steps, warmup, estimator=0, headline=False, clocks=False, prebuilt=None, dump=None):
     """One render workload (C1-C4) at ctx.world GPUs: device-timed value, e2e through the public API with host buffers,
-    hashes of the reduced buffer and of the frame, per-kernel roofline (rank 0)."""
+    hashes of the reduced buffer and of the frame, per-kernel roofline (rank 0). dump: directory that receives what the
+    last timed step returned to the caller (rank 0): the reduced accumulation buffer (int64 fixed point, 2^32 per unit,
+    as float64) and the RGB8 frame (as float32), each (pixels, 3), for a seeded sample of pixels (pixel_index.npy)."""
     import hashlib
     import numpy as np
     import cudaraytracing_b200 as crt
@@ -334,6 +363,11 @@ def render_workload(ctx, name, steps, warmup, estimator=0, headline=False, clock
         # identity of the result: the reduced fixed-point buffer and the tone-mapped frame do not depend on the number of
         # GPUs, the pool size or the scheduling (DESIGN.md section 6) - these two hashes must be equal at N = 1, 2, 4, 8
         acc = render.get_accum_i64()
+        if dump:
+            idx = dump_sample_index(npix, 3 * 8 + 3 * 4 + 8)
+            dump_outputs(dump, {"pixel_index": idx.astype(np.float64),
+                                "accum": acc.reshape(npix, 3)[idx].astype(np.float64),
+                                "frame": frame_np.reshape(npix, 3)[idx].astype(np.float32)})
         out = {
             "value": round(total_samples * steps / (ms_dev * 1e3), 2), "unit": "Msamples/s", "ms_per_step": round(ms_dev / steps, 4),
             "e2e": {"value": round(total_samples * steps / (max(ms_e2e, wall_e2e) * 1e3), 2), "unit": "Msamples/s", "h2d_bytes_per_step": 13 * 4,
@@ -411,15 +445,15 @@ def render_workload(ctx, name, steps, warmup, estimator=0, headline=False, clock
 
 def ours(args):
     ctx = Ctx(args)
-    main = render_workload(ctx, args.workload, args.steps, args.warmup, estimator=args.estimator, headline=True, clocks=True)
+    main = render_workload(ctx, args.workload, args.steps, args.warmup, estimator=args.estimator, headline=True, clocks=True,
+                           dump=args.dump_outputs)
     subs = {}
     if args.workload == "c3" and not args.no_sub:
-        # the other BASELINE configs, short, at the same number of GPUs (the shipped configs take milliseconds)
-        k = max(args.steps, 5)
-        subs["c1"] = render_workload(ctx, "c1", k, 3)
-        subs["c2"] = render_workload(ctx, "c2", k, 3)
-        subs["c2_mis"] = render_workload(ctx, "c2", k, 3, estimator=1)
-        subs["c5"], subs["c4"] = c5_workload(ctx, max(1, min(args.steps, 3)), 3, with_c4=True)
+        # the other BASELINE configs at the same number of GPUs and the same number of timed steps
+        subs["c1"] = render_workload(ctx, "c1", args.steps, 3)
+        subs["c2"] = render_workload(ctx, "c2", args.steps, 3)
+        subs["c2_mis"] = render_workload(ctx, "c2", args.steps, 3, estimator=1)
+        subs["c5"], subs["c4"] = c5_workload(ctx, args.steps, 3, with_c4=True)
     if ctx.rank == 0:
         out = {"metric": "Msamples/s", "value": main["value"], "unit": "Msamples/s", "n_gpus": ctx.world, "steps": args.steps, "warmup": args.warmup,
                "ms_per_step": main["ms_per_step"], "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32",
@@ -531,9 +565,10 @@ def ref_render_workload(ref, name, steps, warmup, spp_list):
                         "cpu": cpu_model()}}
 
 
-def ref_synthetic_child(grid_n, n_rays, spp, out_path):
+def ref_synthetic_child(grid_n, n_rays, spp, out_path, steps=3, warmup=1):
     """Runs in a child process (the parent enforces the time limit): the reference's host BVH build over the synthetic scene,
-    its DeviceBVH::intersect on C5 rays (ref_trace) and its render kernel on the C4 camera."""
+    its DeviceBVH::intersect on C5 rays (ref_trace; best kernel time of `steps` timed calls) and its render kernel on the C4
+    camera (mean of `steps` timed calls); `warmup` untimed calls before each."""
     import numpy as np
     from tools import synthetic as sy
     ref = RefLib()
@@ -570,12 +605,13 @@ def ref_synthetic_child(grid_n, n_rays, spp, out_path):
     t = np.zeros(n_rays, np.float32)
     kms = C.c_float()
     best = 1e30
-    for _ in range(3):
+    for k in range(warmup + steps):
         if R.ref_trace(h, rays.ctypes.data, n_rays, t.ctypes.data, C.byref(kms)) != 0:
             res["c5"] = "ref_trace failed"
             save()
             return
-        best = min(best, kms.value)
+        if k >= warmup:
+            best = min(best, kms.value)
     res["c5"] = {"value": round(n_rays / best / 1e3, 2), "unit": "Mrays/s", "rays": n_rays, "kernel_ms": round(best, 3),
                  "hit_frac": round(float((t < 1e30).mean()), 4),
                  "what": "DeviceBVH::intersect (DeviceBVH.cuh:128-170), one thread per ray, closest hit; the reference has no any-hit traversal "
@@ -588,19 +624,19 @@ def ref_synthetic_child(grid_n, n_rays, spp, out_path):
     frame = np.zeros(W * H * 3, np.uint8)
     wms = C.c_double()
     ws = []
-    for k in range(3):
+    for k in range(warmup + steps):
         if R.ref_render(h, eye.ctypes.data, M.ctypes.data, float(fovy), spp, float(cam["P_RR"]), int(cam["light_sample_n"]), frame.ctypes.data,
                         C.byref(kms), C.byref(wms)) != 0:
             res["c4"] = "ref_render failed"
             save()
             return
-        if k:
+        if k >= warmup:
             ws.append(wms.value)
     res["c4"] = {"value": round(W * H * spp * len(ws) / (sum(ws) * 1e3), 3), "unit": "Msamples/s", "spp_timed": spp, "ms_per_step": round(sum(ws) / len(ws), 2)}
     save()
 
 
-def ref_synthetic_workload(limit_s):
+def ref_synthetic_workload(limit_s, steps=3, warmup=1):
     """C4 / C5 reference numbers (BASELINE.md section 3): the full 10M-triangle scene under a time limit ("DNF > T" if its host
     build does not finish), and when it does not, the largest grid of the ladder that does."""
     import subprocess
@@ -608,7 +644,7 @@ def ref_synthetic_workload(limit_s):
     out = {}
     for grid_n in (sy.C4_FULL_N, 1001, 513):
         path = os.path.join(tempfile.mkdtemp(prefix="crt_ref_"), "res.json")
-        code = "import bench; bench.ref_synthetic_child(%d, %d, %d, %r)" % (grid_n, 2000000, 4, path)
+        code = "import bench; bench.ref_synthetic_child(%d, %d, %d, %r, %d, %d)" % (grid_n, 2000000, 4, path, steps, warmup)
         t0 = time.time()
         try:
             subprocess.run([sys.executable, "-c", code], cwd=ROOT, timeout=limit_s, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
@@ -639,7 +675,7 @@ def reference(args):
         print(json.dumps({"impl": "reference", "unavailable": str(e)}))
         return
     if WORKLOADS[args.workload][0] == "synthetic":
-        r = ref_synthetic_workload(args.ref_limit)
+        r = ref_synthetic_workload(args.ref_limit, args.steps, args.warmup)
         done = [v for v in r.values() if "c5" in v and isinstance(v["c5"], dict)]
         key = "c5" if args.workload == "c5" else "c4"
         if not done or not isinstance(done[-1].get(key), dict):
@@ -647,7 +683,7 @@ def reference(args):
             return
         d = done[-1]
         print(json.dumps({"impl": "reference", "metric": "Mrays/s (closest-hit)" if key == "c5" else "Msamples/s", "value": d[key]["value"],
-                          "unit": d[key]["unit"], "n_gpus": 1, "steps": 3, "warmup": 1, "ms_per_step": d[key].get("kernel_ms", d[key].get("ms_per_step")),
+                          "unit": d[key]["unit"], "n_gpus": 1, "steps": args.steps, "warmup": args.warmup, "ms_per_step": d[key].get("kernel_ms", d[key].get("ms_per_step")),
                           "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": DATA_NOTE["synthetic"],
                           "config": {"workload": WORKLOADS[args.workload][4], "triangles": d["triangles"], "grid_n": d["grid_n"]},
                           "e2e": {"value": d[key]["value"], "unit": d[key]["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -666,9 +702,9 @@ def reference(args):
         return
     subs = {}
     if args.workload == "c3" and not args.no_sub:
-        subs["c1"] = ref_render_workload(ref, "c1", max(args.steps, 5), 3, [1 << 30])
-        subs["c2"] = ref_render_workload(ref, "c2", max(args.steps, 5), 3, [1 << 30])
-        syn = ref_synthetic_workload(args.ref_limit)
+        subs["c1"] = ref_render_workload(ref, "c1", args.steps, 3, [1 << 30])
+        subs["c2"] = ref_render_workload(ref, "c2", args.steps, 3, [1 << 30])
+        syn = ref_synthetic_workload(args.ref_limit, args.steps, args.warmup)
         done = [v for v in syn.values() if isinstance(v.get("c5"), dict)]
         subs["c5"] = dict(done[-1]["c5"], triangles=done[-1]["triangles"], grid_n=done[-1]["grid_n"],
                           host_bvh_build_ms=done[-1]["host_bvh_build_ms"]) if done else {"unavailable": "see synthetic"}
@@ -686,10 +722,12 @@ def reference(args):
     print(json.dumps(out), flush=True)
 
 
-def c5_workload(ctx, steps, warmup, n_total=None, with_c4=False):
+def c5_workload(ctx, steps, warmup, n_total=None, with_c4=False, dump=None):
     """C5: 100M incoherent rays against the 10M-triangle BVH; closest-hit and any-hit Mrays/s with the rays resident in HBM, and
     the same through crt_trace_rays with HOST buffers (rays H2D, hits D2H inside the timed call). Rays are independent: they
-    are sharded over the ranks, no collective."""
+    are sharded over the ranks, no collective. dump: directory that receives, for a seeded sample of rank 0's rays
+    (ray_index.npy), the hit distance (float32) and face id (float64, -1 on a miss) of the last timed closest-hit and
+    any-hit steps. An any-hit ray reports one of its blockers, and which one depends on scheduling: compare any_face >= 0."""
     import hashlib
     import numpy as np
     import cudaraytracing_b200 as crt
@@ -703,6 +741,11 @@ def c5_workload(ctx, steps, warmup, n_total=None, with_c4=False):
     t_out = torch.empty(n, dtype=torch.float32, device=ctx.dev)
     f_out = torch.empty(n, dtype=torch.int32, device=ctx.dev)
     res = {}
+    dumped = {}
+    if dump and ctx.rank == 0:
+        idx = dump_sample_index(n, 2 * (4 + 8) + 8)
+        dumped["ray_index"] = (idx + n0).astype(np.float64)
+        idx_dev = torch.from_numpy(idx).to(ctx.dev)
     for mode, name in ((crt.RAY_CLOSEST, "closest"), (crt.RAY_ANY, "any")):
         scene.random_rays_device(rays.data_ptr(), n, start=n0, key=0xC5, any_hit=(mode == crt.RAY_ANY), stream=ctx.stream.cuda_stream)
         for _ in range(warmup):
@@ -719,6 +762,11 @@ def c5_workload(ctx, steps, warmup, n_total=None, with_c4=False):
         head = min(n, 1000000)
         digest = hashlib.sha256(t_out[:head].cpu().numpy().tobytes() + f_out[:head].cpu().numpy().tobytes()).hexdigest()
         res[name] = dict(ms=kms / steps, mrays=n_total * steps / (kms * 1e3), hit_frac=hits / n, sha=digest)
+        if dumped:
+            dumped[name + "_t"] = t_out[idx_dev].cpu().numpy().astype(np.float32)
+            dumped[name + "_face"] = f_out[idx_dev].cpu().numpy().astype(np.float64)
+    if dumped:
+        dump_outputs(dump, dumped)
     # e2e: host buffers through crt_trace_rays (pinned staging, chunks on two streams inside the library)
     nb = min(n, int(os.environ.get("CRT_C5_E2E_RAYS", "20000000")))
     scene.random_rays_device(rays.data_ptr(), nb, start=n0, key=0xC5, any_hit=False, stream=ctx.stream.cuda_stream)
@@ -731,7 +779,7 @@ def c5_workload(ctx, steps, warmup, n_total=None, with_c4=False):
     for _ in range(max(1, min(warmup, 2))):               # warm-up at full size: chunk buffers, first touch of the result pages
         scene.trace_rays(host_rays, crt.RAY_CLOSEST, out=(pin_t.numpy(), pin_f.numpy()))
     ctx.barrier()
-    e2e_calls = max(1, min(steps, 3))
+    e2e_calls = steps
     t0 = time.time()
     for _ in range(e2e_calls):
         ht, hf, _ = scene.trace_rays(host_rays, crt.RAY_CLOSEST, out=(pin_t.numpy(), pin_f.numpy()))
@@ -740,8 +788,9 @@ def c5_workload(ctx, steps, warmup, n_total=None, with_c4=False):
     page_t, page_f = np.zeros(len(pageable), np.float32), np.zeros(len(pageable), np.int32)
     scene.trace_rays(pageable, crt.RAY_CLOSEST, out=(page_t, page_f))
     t0 = time.time()
-    scene.trace_rays(pageable, crt.RAY_CLOSEST, out=(page_t, page_f))
-    pageable_s = ctx.allmax([time.time() - t0])[0]
+    for _ in range(steps):
+        scene.trace_rays(pageable, crt.RAY_CLOSEST, out=(page_t, page_f))
+    pageable_s = ctx.allmax([(time.time() - t0) / steps])[0]
     out = None
     if ctx.rank == 0:
         peaks, peak_kind = load_peaks()
@@ -798,7 +847,7 @@ def c5_workload(ctx, steps, warmup, n_total=None, with_c4=False):
         # C4: the 1920x1080 spp 64 frame of the same 10M-triangle scene (no second build of scene or oracle tree)
         c4cfg = Workload("c4")
         c4cfg._arrays = cfg._arrays
-        c4 = render_workload(ctx, "c4", max(1, min(steps, 3)), 2, prebuilt=(c4cfg, scene, build_ms) + ((O,) if ctx.rank == 0 else ()))
+        c4 = render_workload(ctx, "c4", steps, 2, prebuilt=(c4cfg, scene, build_ms) + ((O,) if ctx.rank == 0 else ()))
     del scene
     return (out, c4) if with_c4 else out
 
@@ -808,7 +857,7 @@ def ours_c5(args):
     sampler = ClockSampler(ctx.local) if ctx.rank == 0 else None
     if sampler:
         sampler.start()
-    r = c5_workload(ctx, args.steps, args.warmup)
+    r = c5_workload(ctx, args.steps, args.warmup, dump=args.dump_outputs)
     if ctx.rank == 0:
         out = {"metric": r.pop("metric"), "value": r.pop("value"), "unit": r.pop("unit"), "n_gpus": ctx.world, "steps": args.steps, "warmup": args.warmup,
                "ms_per_step": r.pop("ms_per_step"), "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32",
@@ -832,7 +881,7 @@ def cpu_model():
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3, help="timed steps of every measurement")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c3", choices=sorted(WORKLOADS))
@@ -841,7 +890,14 @@ def main():
     ap.add_argument("--ref-limit", type=int, default=240, help="reference arm, synthetic scene: seconds before its host build is DNF")
     ap.add_argument("--estimator", type=int, default=0, choices=[0, 1], help="0 compat (the reference's estimator), 1 mis")
     ap.add_argument("--no-sub", action="store_true", help="default C3 run: skip the short C1 / C2 / C5 sub-measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the headline workload's last step returned as DIR/<name>.npy "
+                         "(float32 / float64, at most 64 MB, a seeded sample of larger outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the ours arm's outputs")
     if args.builder:
         os.environ["CRT_BUILDER"] = args.builder
     if args.impl == "reference":

@@ -47,6 +47,23 @@ def test_cpu_baseline_leg_counts_visits_on_the_same_tree(builder, monkeypatch):
         assert per_ray["closest_inner"] < 0.6 * pr2["closest_inner"]
 
 
+def test_dump_sample_is_seeded_and_bounded(tmp_path):
+    small = bench.dump_sample_index(1000, 44)
+    assert np.array_equal(small, np.arange(1000))                # fits: every item
+    npix = 3840 * 2160
+    a, b = bench.dump_sample_index(npix, 44), bench.dump_sample_index(npix, 44)
+    assert np.array_equal(a, b) and len(a) * 44 <= bench.DUMP_BYTES and len(a) > npix // 8
+    assert np.all(np.diff(a) > 0) and a[0] >= 0 and a[-1] < npix
+    full = {"pixel_index": a.astype(np.float64), "accum": np.zeros((len(a), 3)), "frame": np.zeros((len(a), 3), np.float32)}
+    bench.dump_outputs(str(tmp_path / "full"), full)            # the C3 dump, headers included, within the budget
+    assert sum(os.path.getsize(tmp_path / "full" / (k + ".npy")) for k in full) <= 64 * 10 ** 6
+    bench.dump_outputs(str(tmp_path / "d"), {"x": np.ones(7, np.float32), "i": a[:5].astype(np.float64)})
+    assert np.array_equal(np.load(tmp_path / "d" / "x.npy"), np.ones(7, np.float32))
+    assert np.array_equal(np.load(tmp_path / "d" / "i.npy"), a[:5])
+    with pytest.raises(AssertionError):
+        bench.dump_outputs(str(tmp_path / "e"), {"x": np.ones(7, np.int64)})
+
+
 def test_reference_arm_runs_on_rank_zero_only(monkeypatch, capsys):
     import argparse
     monkeypatch.setenv("RANK", "1")
