@@ -191,8 +191,21 @@ CRT_DEV bool tri_test(V3 v1, V3 e1, V3 e2, V3 o, V3 d, float* t_out) {
     return 0.0f < alpha && alpha < 1.0f && 0.0f < beta && beta < 1.0f && 0.0f < gamma && gamma < 1.0f;
 }
 
+// Direction components below kParallelDir = 2^-40 in magnitude count as parallel in the box tests (box_inv gives them a
+// NaN inverse); the triangle test keeps the true direction. The threshold is set by overflow alone:
+//  * below 2^-128, 1/d overflows to inf, and a ray starting in a box plane got 0 * inf = NaN on one plane and +-inf on the
+//    other, an empty slab; in the wide node step (crt_wide.cuh) b = s / d made the folded bias fma(-32768, b, a) overflow
+//    to -inf once |d| < ~s * 2^-113 (s: the node's cell size), which culled every child of the node;
+//  * above 2^-40, |1/d| <= 2^40: for coordinates and origins within +-2^72 (the range crt.h states) a node spans at most
+//    2^73, its cell size is s <= 2^66, the folded bias 32768 * s / d <= 2^121, a = (p - o) / d <= 2^113 and the pair
+//    slab's plane distances likewise <= 2^113 - below FLT_MAX ~ 2^128;
+//  * treating a component below 2^-40 as parallel stays conservative: up to the exit distance texit the ray moves at most
+//    2^-40 * texit along the axis, less than one rounding (2^-24 relative) of parallel_ok's margin, which holds
+//    2^-17 * texit. Exact zeros therefore keep the margin they had.
+static constexpr float kParallelDir = 9.094947017729282379e-13f;      // 2^-40
+
 // Conservative slab test (DESIGN.md "Traversal rule"). NaN plane distances drop out of fminf / fmaxf.
-// Axis the ray is parallel to (direction component exactly 0, inverse = NaN - box_inv below): its plane distances
+// Axis the ray is parallel to (direction component below kParallelDir, inverse = NaN - box_inv below): its plane distances
 // drop out of the min/max of the slab test, and the axis is tested here instead: o must lie in [lo, hi] widened by
 // 2^-17 * (|o| + exit distance + summed box extent). Statement and rationale: oracle/orc_bvh.cpp parallel_ok.
 CRT_DEV bool parallel_ok(float lo, float hi, float o, float texit, float ext) {
@@ -210,7 +223,12 @@ CRT_DEV bool slab(float lox, float hix, float loy, float hiy, float loz, float h
     float tmin = fmaxf(fmaxf(fminf(tx0, tx1), fminf(ty0, ty1)), fmaxf(fminf(tz0, tz1), 0.0f));
     float tmax = fminf(fminf(fmaxf(tx0, tx1), fmaxf(ty0, ty1)), fminf(fmaxf(tz0, tz1), limit));
     *enter = tmin;
-    bool hit = tmin <= tmax * kSlabSlack;
+    // absolute slack: 2^-21 * the largest plane distance, as in the wide node step (statement: oracle/orc_bvh.cpp slab).
+    // Without it a ray leaving a box plane (o.y == hi.y, d.y > 0) exits that slab at t = 0 exactly, the relative slack is 0,
+    // and the hits the triangle test accepts just past the box's edge in that plane were lost, for any size of d.y.
+    const float pad = fmaxf(fmaxf(fmaxf(fabsf(tx0), fabsf(tx1)), fmaxf(fabsf(ty0), fabsf(ty1))),
+                            fmaxf(fabsf(tz0), fabsf(tz1))) * 4.76837158203125e-07f;
+    bool hit = tmin <= fmaf(tmax, kSlabSlack, pad);
     if (zray && hit) {
         const float ext = ((hix - lox) + (hiy - loy)) + (hiz - loz);
         if (inv.x != inv.x) hit = parallel_ok(lox, hix, o.x, tmax, ext);
@@ -220,14 +238,14 @@ CRT_DEV bool slab(float lox, float hix, float loy, float hiy, float loz, float h
     return hit;
 }
 
-// Inverse direction for the box tests: 1/d, and NaN for a component that is exactly zero, so that this axis never
-// culls (every plane distance on it is NaN and drops out of fminf / fmaxf). With 1/0 = inf a ray lying IN a box
-// plane (o.x == plane) gave 0 * inf = NaN on that plane and +-inf on the other, min(NaN, +inf) = +inf emptied the
-// slab, and the traversal dropped boxes whose triangles the Moeller-Trumbore test accepts; the same happens when the
-// origin (a computed hit point) sits one ulp outside a box whose triangle still passes the test. Exact zeros are not
-// rare: sincos_2pi is exact at the quadrants. Found by the wide-node render (profiles/r01_s12_wide_vs_pair.md).
-// Statement: oracle/orc_math.h box_inv.
-CRT_DEV float box_inv(float x) { return x == 0.0f ? __int_as_float(0x7fc00000) : 1.0f / x; }
+// Inverse direction for the box tests: 1/d, and NaN for a component below kParallelDir in magnitude (zero included), so
+// that this axis never culls (every plane distance on it is NaN and drops out of fminf / fmaxf) and parallel_ok tests it
+// instead. With 1/0 = inf a ray lying IN a box plane (o.x == plane) gave 0 * inf = NaN on that plane and +-inf on the
+// other, min(NaN, +inf) = +inf emptied the slab, and the traversal dropped boxes whose triangles the Moeller-Trumbore
+// test accepts; the same happens when the origin (a computed hit point) sits one ulp outside a box whose triangle still
+// passes the test. Exact zeros are not rare: sincos_2pi is exact at the quadrants. Found by the wide-node render
+// (profiles/r01_s12_wide_vs_pair.md); tiny non-zero components: kParallelDir above. Statement: oracle/orc_math.h box_inv.
+CRT_DEV float box_inv(float x) { return fabsf(x) < kParallelDir ? __int_as_float(0x7fc00000) : 1.0f / x; }
 CRT_DEV V3 box_inv3(V3 d) { return mk3(box_inv(d.x), box_inv(d.y), box_inv(d.z)); }
 
 struct HitRec { float t; int slot; int face; };

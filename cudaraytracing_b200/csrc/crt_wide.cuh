@@ -44,7 +44,7 @@ struct WideStep {
     uint32_t child_base, tri_base, meta_lo, meta_hi, imask;
 };
 
-// Rays with a parallel axis (direction component exactly 0, NaN inverse; rare): the children that passed the slab test
+// Rays with a parallel axis (direction component below kParallelDir, NaN inverse - box_inv; rare): the children that passed the slab test
 // are tested on those axes by parallel_ok. Out of line, so that the common path carries no branch per child.
 // The node is read again here (L1) rather than handed over in sixteen registers that would stay live across the child tests.
 static __device__ __noinline__ uint32_t wide_parallel_filter(const uint4* __restrict__ p, V3 o, V3 inv, float lim, uint32_t hits) {

@@ -119,6 +119,10 @@ int crt_config_load(const char* json_path, crt_config* out);
 int crt_inverse_view_matrix(const float eye[3], const float lookat[3], const float up[3], float out9[9]);
 
 /* ---- scene ----------------------------------------------------------------------------- */
+/* Coordinate range: for vertex coordinates and ray origins within +-2^72 no term of the traversal's box tests can
+ * overflow, whatever the ray direction (derivation: csrc/crt_device.cuh kParallelDir), so the hits equal a brute-force
+ * test of every triangle. Ingest refuses only non-finite coordinates; beyond 2^72 a box test can lose hits. The triangle
+ * test itself multiplies three lengths, so triangles and distances beyond ~2^42 overflow in it. */
 /* Scene::Scene, include/Scene.h:28 (width/height live on the render handle here). */
 int crt_scene_create(crt_scene** out);
 /* Loader::read_OBJ + the load_object / add_normal_obj / add_light_obj loop, src/main.cu:122-145,

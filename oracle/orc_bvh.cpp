@@ -428,8 +428,9 @@ void build_new_bvh(const Scene& s, unsigned thresh_n, int builder, NewBVH& out) 
 // New traversal rule (DESIGN.md §"Traversal rule"): conservative slabs, near child first,
 // far child pushed, leaves postponed on the stack; t-culling against 1.0001 * current limit.
 // =============================================================================================
-// A direction component that is exactly zero has a NaN inverse (orc_math.h box_inv), so its plane distances drop out
-// of the min/max above; the axis is tested here instead: the ray stays at o on it, so o must lie inside [lo, hi],
+// A direction component below kParallelDir (2^-40, zero included) has a NaN inverse (orc_math.h box_inv), so its plane
+// distances drop out of the min/max above; the axis is tested here instead: the ray stays at o on it (to within
+// 2^-40 * exit distance, less than one rounding of dlt), so o must lie inside [lo, hi],
 // widened by 2^-17 * (|o| + exit distance + box extent summed over the axes) - the same relative slack as kSlabSlack,
 // applied sideways: o is a computed hit point (a few ulp off its surface) and the triangle test's acceptance band scales
 // with the distance AND with the triangle's size (a ray 3e-5 outside the 556-unit ceiling triangle of cornell-box is
@@ -450,7 +451,14 @@ static inline bool slab(float lox, float hix, float loy, float hiy, float loz, f
     float tmin = fmaxf(fmaxf(fminf(tx0, tx1), fminf(ty0, ty1)), fmaxf(fminf(tz0, tz1), 0.0f));
     float tmax = fminf(fminf(fmaxf(tx0, tx1), fmaxf(ty0, ty1)), fminf(fmaxf(tz0, tz1), limit));
     *enter = tmin;
-    if (!(tmin <= tmax * kSlabSlack)) return false;
+    // Absolute slack pad = 2^-21 * the largest plane distance, as in the wide node step (wide8_intersect). The relative
+    // slack is 0 when tmax is: a ray leaving a box plane (o.y == hi.y, d.y > 0) exits that slab at t = 0 exactly, but the
+    // triangle test accepts hits a little past the edge that lies in that plane (a ray from the ceiling hitting a wall
+    // 2e-5 away). The pad is 2^-21 * |plane - o| / |d| on the axis that gives the largest distance: in position along
+    // that axis, a band of at least 2^-22 of the box's extent.
+    const float pad = fmaxf(fmaxf(fmaxf(fabsf(tx0), fabsf(tx1)), fmaxf(fabsf(ty0), fabsf(ty1))),
+                            fmaxf(fabsf(tz0), fabsf(tz1))) * 4.76837158203125e-07f;
+    if (!(tmin <= fmaf(tmax, kSlabSlack, pad))) return false;
     // axes the ray is parallel to (inverse = NaN, see box_inv): the origin coordinate must lie in the box's interval
     if (inv.x != inv.x || inv.y != inv.y || inv.z != inv.z) {
         const float ext = ((hix - lox) + (hiy - loy)) + (hiz - loz);

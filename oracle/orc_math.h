@@ -52,11 +52,15 @@ static inline V3 normalize_rcp(V3 a) {
     if (n > 0.0f) return a * (1.0f / sqrtf(n));
     return a;
 }
-// Inverse direction for the box tests of the new traversal rules: 1/d, NaN for a component that is exactly zero, so
-// that this axis never culls (NaN plane distances drop out of fminf / fmaxf). With 1/0 = inf a ray lying in a box plane
-// made the pair-node slab empty (min(0 * inf, +inf) = +inf) and boxes were dropped whose triangles pass the triangle
-// test. The reference rule (ref_intersect) keeps the reference's plain 1/d (Ray.cuh:14).
-static inline float box_inv(float x) { return x == 0.0f ? std::numeric_limits<float>::quiet_NaN() : 1.0f / x; }
+// Inverse direction for the box tests of the new traversal rules: 1/d, NaN for a component whose magnitude is below
+// kParallelDir (zero included), so that this axis never culls (NaN plane distances drop out of fminf / fmaxf) and is
+// tested by parallel_ok (orc_bvh.cpp) instead. With 1/0 = inf a ray lying in a box plane made the pair-node slab empty
+// (min(0 * inf, +inf) = +inf) and boxes were dropped whose triangles pass the triangle test; small non-zero components
+// lost hits too (1/d overflowing, the wide node step's folded bias overflowing). Choice of the threshold and its bounds:
+// crt_device.cuh kParallelDir. The triangle test keeps the true direction. The reference rule (ref_intersect) keeps the
+// reference's plain 1/d (Ray.cuh:14).
+static const float kParallelDir = 9.094947017729282379e-13f;      // 2^-40
+static inline float box_inv(float x) { return fabsf(x) < kParallelDir ? std::numeric_limits<float>::quiet_NaN() : 1.0f / x; }
 static inline V3 vmin(V3 a, V3 b) { return V3{fminf(a.x, b.x), fminf(a.y, b.y), fminf(a.z, b.z)}; }
 static inline V3 vmax(V3 a, V3 b) { return V3{fmaxf(a.x, b.x), fmaxf(a.y, b.y), fmaxf(a.z, b.z)}; }
 
