@@ -13,7 +13,7 @@ using namespace crt;
 struct crt_scene {
     HostScene host;
     DeviceScene dev;
-    RayBatcher* batcher = nullptr;
+    RayBatcherPtr batcher;
     uint32_t scene_hash = 0;            // identity of the built scene (checkpoints), 0 = not built
     bool built = false;
     uint32_t thresh_n = 0;
@@ -21,13 +21,13 @@ struct crt_scene {
 
 struct crt_render {
     crt_scene* scene = nullptr;
-    Wavefront* wf = nullptr;
+    WavefrontPtr wf;
     RenderSettings rs;
+    Stream own_stream;                  // the render's own stream, until crt_render_set_stream replaces it
     cudaStream_t stream = nullptr;
-    bool own_stream = false;
     bool rendered = false;
-    float* d_linear = nullptr;
-    uint8_t* d_rgb8 = nullptr;
+    DevBuf<float> d_linear;
+    DevBuf<uint8_t> d_rgb8;
     crt_render_stats stats{};
     // camera of the last run_view (or of the loaded checkpoint): what the accumulation buffer belongs to
     bool cam_set = false;
@@ -189,11 +189,11 @@ int crt_scene_build_bvh(crt_scene* s, uint32_t thresh_n, int builder, int device
     int n = crt_device_count();
     if (n <= 0) { set_error("crt_scene_build_bvh: no CUDA device (there is no CPU fallback)"); return CRT_ERR_CUDA; }
     CHECK_ARG(device >= 0 && device < n, "crt_scene_build_bvh: device out of range");
-    if (s->batcher) { ray_batcher_destroy(s->batcher); s->batcher = nullptr; }       // its buffers belong to the previous build's device
+    s->batcher.reset();                                                              // its buffers belong to the previous build's device
     int rc = upload_scene(s->host, thresh_n, builder, device, s->dev, build_ms);
     s->built = rc == CRT_OK;
     s->thresh_n = thresh_n;
-    if (rc != CRT_OK) { s->dev.release(); return rc; }                               // nothing half-uploaded stays behind
+    if (rc != CRT_OK) { s->dev = DeviceScene(); return rc; }                         // nothing half-uploaded stays behind
     // identity of the scene for checkpoints: triangle count, leaf rule and an FNV-1a of the vertex and material tables
     {
         uint64_t h = fnv1a64(s->host.verts.data(), s->host.verts.size() * sizeof(float) / 8 * 8);
@@ -270,9 +270,9 @@ int crt_scene_export_bvh(crt_scene* s, crt_bvh_node* nodes, int32_t* tri_order, 
     if (!s->built) { set_error("crt_scene_export_bvh: BVH not built"); return CRT_ERR_STATE; }
     if (s->dev.wide) { set_error("crt_scene_export_bvh: the scene has 8-wide nodes (use crt_scene_export_bvh8)"); return CRT_ERR_STATE; }
     CRT_CUDA(cudaSetDevice(s->dev.device));
-    if (nodes && s->dev.n_nodes) CRT_CUDA(cudaMemcpy(nodes, s->dev.nodes, sizeof(crt_bvh_node) * s->dev.n_nodes, cudaMemcpyDeviceToHost));
-    if (tri_order && s->dev.n_tris) CRT_CUDA(cudaMemcpy(tri_order, s->dev.order, sizeof(int32_t) * s->dev.n_tris, cudaMemcpyDeviceToHost));
-    if (last && s->dev.n_tris) CRT_CUDA(cudaMemcpy(last, s->dev.last, s->dev.n_tris, cudaMemcpyDeviceToHost));
+    if (nodes && s->dev.n_nodes) CRT_CUDA(cudaMemcpy(nodes, s->dev.nodes.get(), sizeof(crt_bvh_node) * s->dev.n_nodes, cudaMemcpyDeviceToHost));
+    if (tri_order && s->dev.n_tris) CRT_CUDA(cudaMemcpy(tri_order, s->dev.order.get(), sizeof(int32_t) * s->dev.n_tris, cudaMemcpyDeviceToHost));
+    if (last && s->dev.n_tris) CRT_CUDA(cudaMemcpy(last, s->dev.last.get(), s->dev.n_tris, cudaMemcpyDeviceToHost));
     if (bounds) memcpy(bounds, s->dev.bounds, sizeof(float) * 6);
     return CRT_OK;
     });
@@ -285,9 +285,9 @@ int crt_scene_export_bvh8(crt_scene* s, crt_bvh8_node* nodes, int32_t* tri_order
     if (!s->built) { set_error("crt_scene_export_bvh8: BVH not built"); return CRT_ERR_STATE; }
     if (!s->dev.wide) { set_error("crt_scene_export_bvh8: the scene has child-pair nodes (use crt_scene_export_bvh)"); return CRT_ERR_STATE; }
     CRT_CUDA(cudaSetDevice(s->dev.device));
-    if (nodes && s->dev.n_nodes) CRT_CUDA(cudaMemcpy(nodes, s->dev.nodes, sizeof(crt_bvh8_node) * s->dev.n_nodes, cudaMemcpyDeviceToHost));
-    if (tri_order && s->dev.n_tris) CRT_CUDA(cudaMemcpy(tri_order, s->dev.order, sizeof(int32_t) * s->dev.n_tris, cudaMemcpyDeviceToHost));
-    if (last && s->dev.n_tris) CRT_CUDA(cudaMemcpy(last, s->dev.last, s->dev.n_tris, cudaMemcpyDeviceToHost));
+    if (nodes && s->dev.n_nodes) CRT_CUDA(cudaMemcpy(nodes, s->dev.nodes.get(), sizeof(crt_bvh8_node) * s->dev.n_nodes, cudaMemcpyDeviceToHost));
+    if (tri_order && s->dev.n_tris) CRT_CUDA(cudaMemcpy(tri_order, s->dev.order.get(), sizeof(int32_t) * s->dev.n_tris, cudaMemcpyDeviceToHost));
+    if (last && s->dev.n_tris) CRT_CUDA(cudaMemcpy(last, s->dev.last.get(), s->dev.n_tris, cudaMemcpyDeviceToHost));
     if (bounds) memcpy(bounds, s->dev.bounds, sizeof(float) * 6);
     return CRT_OK;
     });
@@ -305,7 +305,7 @@ int crt_scene_bvh_kind(crt_scene* s, int* builder) {
 int crt_scene_destroy(crt_scene* s) {
     return guarded("crt_scene_destroy", [&]() -> int {
     if (!s) return CRT_OK;
-    if (s->built) { cudaSetDevice(s->dev.device); ray_batcher_destroy(s->batcher); s->dev.release(); }
+    if (s->built) cudaSetDevice(s->dev.device);
     delete s;
     return CRT_OK;
     });
@@ -314,9 +314,7 @@ int crt_scene_destroy(crt_scene* s) {
 // ---- ray batches ---------------------------------------------------------------------------
 static int scene_batcher(crt_scene* s) {
     if (s->batcher) return CRT_OK;
-    int rc = ray_batcher_create(s->dev, &s->batcher);
-    if (rc != CRT_OK) { ray_batcher_destroy(s->batcher); s->batcher = nullptr; }
-    return rc;
+    return ray_batcher_create(s->dev, s->batcher);
 }
 
 int crt_trace_rays_device(crt_scene* s, const void* d_rays, uint64_t n, int mode, void* d_t_out, void* d_face_out, void* stream,
@@ -329,7 +327,7 @@ int crt_trace_rays_device(crt_scene* s, const void* d_rays, uint64_t n, int mode
     if (n == 0) { if (kernel_ms) *kernel_ms = 0; return CRT_OK; }
     int rc = scene_batcher(s);
     if (rc != CRT_OK) return rc;
-    return trace_rays_device(s->batcher, s->dev, (const float4*)d_rays, n, mode, (float*)d_t_out, (int*)d_face_out, (cudaStream_t)stream, kernel_ms);
+    return trace_rays_device(s->batcher.get(), s->dev, (const float4*)d_rays, n, mode, (float*)d_t_out, (int*)d_face_out, (cudaStream_t)stream, kernel_ms);
     });
 }
 
@@ -342,7 +340,7 @@ int crt_trace_rays(crt_scene* s, const float* rays, uint64_t n, int mode, float*
     if (n == 0) { if (kernel_ms) *kernel_ms = 0; return CRT_OK; }
     int rc = scene_batcher(s);
     if (rc != CRT_OK) return rc;
-    return trace_rays_host(s->batcher, s->dev, rays, n, mode, t_out, face_out, kernel_ms);
+    return trace_rays_host(s->batcher.get(), s->dev, rays, n, mode, t_out, face_out, kernel_ms);
     });
 }
 
@@ -362,20 +360,17 @@ int crt_render_create(crt_scene* s, uint32_t width, uint32_t height, crt_render*
     CHECK_ARG(width > 0 && height > 0 && (uint64_t)width * height <= (1ull << 28), "crt_render_create: bad image size");
     if (!s->built) { set_error("crt_render_create: build the BVH first (crt_scene_build_bvh)"); return CRT_ERR_STATE; }
     CRT_CUDA(cudaSetDevice(s->dev.device));
-    crt_render* r = new (std::nothrow) crt_render();
+    std::unique_ptr<crt_render> r(new (std::nothrow) crt_render());      // released on failure, with the scene's device current
     if (!r) { set_error("out of memory"); return CRT_ERR_NOMEM; }
     r->scene = s;
     r->rs.width = width; r->rs.height = height;
-    int rc = wavefront_create(s->dev, width, height, &r->wf);
-    if (rc == CRT_OK && cudaStreamCreateWithFlags(&r->stream, cudaStreamNonBlocking) != cudaSuccess) rc = cuda_fail(cudaGetLastError(), "cudaStreamCreate");
-    r->own_stream = true;
-    if (rc == CRT_OK) {
-        cudaError_t e = cudaMalloc(&r->d_linear, sizeof(float) * 3 * (size_t)width * height);
-        if (e == cudaSuccess) e = cudaMalloc(&r->d_rgb8, 3 * (size_t)width * height);
-        if (e != cudaSuccess) rc = cuda_fail(e, "cudaMalloc frame buffers");
-    }
-    if (rc != CRT_OK) { crt_render_destroy(r); return rc; }
-    *out = r;
+    int rc = wavefront_create(s->dev, width, height, r->wf);
+    if (rc != CRT_OK) return rc;
+    CRT_CUDA(create(r->own_stream));
+    r->stream = r->own_stream.get();
+    CRT_CUDA(r->d_linear.alloc(3 * (size_t)width * height));
+    CRT_CUDA(r->d_rgb8.alloc(3 * (size_t)width * height));
+    *out = r.release();
     return CRT_OK;
     });
 }
@@ -440,9 +435,8 @@ int crt_render_clear_range(crt_render* r) {
 int crt_render_set_stream(crt_render* r, void* cuda_stream) {
     return guarded("crt_render_set_stream", [&]() -> int {
     CHECK_ARG(r, "crt_render_set_stream: null handle");
-    if (r->own_stream && r->stream) cudaStreamDestroy(r->stream);
+    r->own_stream.reset();
     r->stream = (cudaStream_t)cuda_stream;
-    r->own_stream = false;
     return CRT_OK;
     });
 }
@@ -466,7 +460,7 @@ int crt_render_run_view(crt_render* r, const float eye[3], const float inv_view[
     memcpy(r->cam_eye, eye, sizeof(r->cam_eye)); memcpy(r->cam_M, inv_view, sizeof(r->cam_M)); r->cam_fovy = fovy_rad;
     r->cam_set = true;
     float tan_half = tanf(fovy_rad / 2);                          // Render.cuh:338, evaluated on the host
-    int rc = wavefront_render(r->wf, r->scene->dev, r->rs, eye, inv_view, tan_half, r->stream, &r->stats);
+    int rc = wavefront_render(r->wf.get(), r->scene->dev, r->rs, eye, inv_view, tan_half, r->stream, &r->stats);
     r->rendered = rc == CRT_OK;
     return rc;
     });
@@ -483,7 +477,7 @@ int crt_render_clear_accum(crt_render* r) {
     return guarded("crt_render_clear_accum", [&]() -> int {
     CHECK_ARG(r, "crt_render_clear_accum: null handle");
     CRT_CUDA(cudaSetDevice(r->scene->dev.device));
-    CRT_CUDA(cudaMemsetAsync(wavefront_accum(r->wf), 0, sizeof(int64_t) * 3 * (size_t)r->rs.width * r->rs.height, r->stream));
+    CRT_CUDA(cudaMemsetAsync(wavefront_accum(r->wf.get()), 0, sizeof(int64_t) * 3 * (size_t)r->rs.width * r->rs.height, r->stream));
     CRT_CUDA(cudaStreamSynchronize(r->stream));
     r->cam_set = false;
     return CRT_OK;
@@ -498,7 +492,7 @@ int crt_render_save_checkpoint(crt_render* r, const char* path, uint64_t work_do
     CRT_CUDA(cudaSetDevice(r->scene->dev.device));
     const size_t n = 3 * (size_t)r->rs.width * r->rs.height;
     std::vector<int64_t> buf(n);
-    CRT_CUDA(cudaMemcpy(buf.data(), wavefront_accum(r->wf), sizeof(int64_t) * n, cudaMemcpyDeviceToHost));
+    CRT_CUDA(cudaMemcpy(buf.data(), wavefront_accum(r->wf.get()), sizeof(int64_t) * n, cudaMemcpyDeviceToHost));
     CheckpointHeader h;
     memset(&h, 0, sizeof(h));
     memcpy(h.magic, kCkptMagic, 8);
@@ -552,7 +546,7 @@ int crt_render_load_checkpoint(crt_render* r, const char* path, uint64_t* work_d
     fclose(f);
     if (rc != CRT_OK) return rc;
     CRT_CUDA(cudaSetDevice(r->scene->dev.device));
-    CRT_CUDA(cudaMemcpy(wavefront_accum(r->wf), buf.data(), sizeof(int64_t) * n, cudaMemcpyHostToDevice));
+    CRT_CUDA(cudaMemcpy(wavefront_accum(r->wf.get()), buf.data(), sizeof(int64_t) * n, cudaMemcpyHostToDevice));
     memcpy(r->cam_eye, h.eye, sizeof(h.eye)); memcpy(r->cam_M, h.M, sizeof(h.M)); r->cam_fovy = h.fovy;
     r->cam_set = true;
     r->rs.accumulate = true;
@@ -568,7 +562,7 @@ int crt_render_load_checkpoint(crt_render* r, const char* path, uint64_t* work_d
 int crt_render_device_accum(crt_render* r, void** d_accum) {
     return guarded("crt_render_device_accum", [&]() -> int {
     CHECK_ARG(r && d_accum, "crt_render_device_accum: null argument");
-    *d_accum = wavefront_accum(r->wf);
+    *d_accum = wavefront_accum(r->wf.get());
     return CRT_OK;
     });
 }
@@ -577,7 +571,7 @@ int crt_render_get_accum_i64(crt_render* r, int64_t* out) {
     return guarded("crt_render_get_accum_i64", [&]() -> int {
     CHECK_ARG(r && out, "crt_render_get_accum_i64: null argument");
     CRT_CUDA(cudaSetDevice(r->scene->dev.device));
-    CRT_CUDA(cudaMemcpy(out, wavefront_accum(r->wf), sizeof(int64_t) * 3 * (size_t)r->rs.width * r->rs.height, cudaMemcpyDeviceToHost));
+    CRT_CUDA(cudaMemcpy(out, wavefront_accum(r->wf.get()), sizeof(int64_t) * 3 * (size_t)r->rs.width * r->rs.height, cudaMemcpyDeviceToHost));
     return CRT_OK;
     });
 }
@@ -585,10 +579,10 @@ int crt_render_get_accum_i64(crt_render* r, int64_t* out) {
 static int resolve_to(crt_render* r, float* lin_host, uint8_t* rgb_host) {
     CRT_CUDA(cudaSetDevice(r->scene->dev.device));
     const uint32_t npix = r->rs.width * r->rs.height;
-    int rc = resolve_device(wavefront_accum(r->wf), npix, r->rs.spp, r->d_linear, r->d_rgb8, r->stream);
+    int rc = resolve_device(wavefront_accum(r->wf.get()), npix, r->rs.spp, r->d_linear.get(), r->d_rgb8.get(), r->stream);
     if (rc != CRT_OK) return rc;
-    if (lin_host) CRT_CUDA(cudaMemcpyAsync(lin_host, r->d_linear, sizeof(float) * 3 * (size_t)npix, cudaMemcpyDeviceToHost, r->stream));
-    if (rgb_host) CRT_CUDA(cudaMemcpyAsync(rgb_host, r->d_rgb8, 3 * (size_t)npix, cudaMemcpyDeviceToHost, r->stream));
+    if (lin_host) CRT_CUDA(cudaMemcpyAsync(lin_host, r->d_linear.get(), sizeof(float) * 3 * (size_t)npix, cudaMemcpyDeviceToHost, r->stream));
+    if (rgb_host) CRT_CUDA(cudaMemcpyAsync(rgb_host, r->d_rgb8.get(), 3 * (size_t)npix, cudaMemcpyDeviceToHost, r->stream));
     CRT_CUDA(cudaStreamSynchronize(r->stream));
     return CRT_OK;
 }
@@ -616,7 +610,7 @@ int crt_render_get_rgb8_device(crt_render* r, void* d_rgb8) {
         set_error("crt_render_get_rgb8_device: d_rgb8 is not device memory of the render's device " + std::to_string(r->scene->dev.device));
         return CRT_ERR_INVALID;
     }
-    int rc = resolve_device(wavefront_accum(r->wf), r->rs.width * r->rs.height, r->rs.spp, r->d_linear, (uint8_t*)d_rgb8, r->stream);
+    int rc = resolve_device(wavefront_accum(r->wf.get()), r->rs.width * r->rs.height, r->rs.spp, r->d_linear.get(), (uint8_t*)d_rgb8, r->stream);
     if (rc != CRT_OK) return rc;
     CRT_CUDA(cudaStreamSynchronize(r->stream));
     return CRT_OK;
@@ -643,10 +637,6 @@ int crt_render_destroy(crt_render* r) {
     return guarded("crt_render_destroy", [&]() -> int {
     if (!r) return CRT_OK;
     if (r->scene) cudaSetDevice(r->scene->dev.device);
-    wavefront_destroy(r->wf);
-    cudaFree(r->d_linear);
-    cudaFree(r->d_rgb8);
-    if (r->own_stream && r->stream) cudaStreamDestroy(r->stream);
     delete r;
     return CRT_OK;
     });
@@ -708,18 +698,19 @@ struct crt_group {
     uint32_t width = 0, height = 0;
     std::vector<int> devices;
     std::vector<DeviceScene> replicas;          // [0] unused: GPU 0 renders the scene handle's own tables
-    std::vector<Wavefront*> wf;
-    std::vector<cudaStream_t> streams;
+    std::vector<WavefrontPtr> wf;
+    std::vector<Stream> streams;
     std::vector<ncclComm_t> comms;
     std::vector<crt_render_stats> stats;
     RenderSettings rs;
-    cudaEvent_t ev_r0 = nullptr, ev_r1 = nullptr;
-    cudaEvent_t ev_band[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    cudaStream_t st_resolve = nullptr;          // devices[0]: resolves band c while band c + 1 is being reduced
+    // on devices[0]:
+    Event ev_r0, ev_r1;
+    Event ev_band[kGroupBands];
+    Stream st_resolve;                          // resolves band c while band c + 1 is being reduced
     bool resolved = false;                      // d_linear / d_rgb8 hold the resolved frame of the last run_view
     float reduce_ms = 0;
-    float* d_linear = nullptr;
-    uint8_t* d_rgb8 = nullptr;
+    DevBuf<float> d_linear;
+    DevBuf<uint8_t> d_rgb8;
     bool rendered = false;
     const DeviceScene& scene_of(size_t g) const { return g == 0 ? scene->dev : replicas[g]; }
 };
@@ -730,19 +721,13 @@ int crt_group_destroy(crt_group* g) {
     if (!g) return CRT_OK;
     for (size_t k = 0; k < g->devices.size(); ++k) {
         cudaSetDevice(g->devices[k]);
-        if (k < g->wf.size()) wavefront_destroy(g->wf[k]);
-        if (k < g->streams.size() && g->streams[k]) cudaStreamDestroy(g->streams[k]);
+        if (k < g->wf.size()) g->wf[k].reset();
+        if (k < g->streams.size()) g->streams[k].reset();
         if (k < g->comms.size() && g->comms[k]) g_nccl.CommDestroy(g->comms[k]);
-        if (k > 0 && k < g->replicas.size()) g->replicas[k].release();
+        if (k > 0 && k < g->replicas.size()) g->replicas[k] = DeviceScene();
     }
     if (!g->devices.empty()) cudaSetDevice(g->devices[0]);
-    if (g->ev_r0) cudaEventDestroy(g->ev_r0);
-    if (g->ev_r1) cudaEventDestroy(g->ev_r1);
-    for (cudaEvent_t e : g->ev_band) if (e) cudaEventDestroy(e);
-    if (g->st_resolve) cudaStreamDestroy(g->st_resolve);
-    cudaFree(g->d_linear);
-    cudaFree(g->d_rgb8);
-    delete g;
+    delete g;                                   // what is left lives on devices[0]
     return CRT_OK;
 }
 
@@ -762,8 +747,8 @@ int crt_group_create(crt_scene* s, uint32_t width, uint32_t height, const int* d
     g->scene = s; g->width = width; g->height = height;
     g->devices.assign(devices, devices + n_devices);
     g->replicas.resize(n_devices);
-    g->wf.assign(n_devices, nullptr);
-    g->streams.assign(n_devices, nullptr);
+    g->wf.resize(n_devices);
+    g->streams.resize(n_devices);
     g->comms.assign(n_devices, nullptr);
     g->stats.resize(n_devices);
     g->rs.width = width; g->rs.height = height;
@@ -771,9 +756,9 @@ int crt_group_create(crt_scene* s, uint32_t width, uint32_t height, const int* d
         for (uint32_t k = 0; k < n_devices; ++k) {
             if (k > 0) { int rc = clone_scene(s->dev, devices[k], g->replicas[k]); if (rc != CRT_OK) return rc; }
             CRT_CUDA(cudaSetDevice(devices[k]));
-            int rc = wavefront_create(g->scene_of(k), width, height, &g->wf[k]);
+            int rc = wavefront_create(g->scene_of(k), width, height, g->wf[k]);
             if (rc != CRT_OK) return rc;
-            CRT_CUDA(cudaStreamCreateWithFlags(&g->streams[k], cudaStreamNonBlocking));
+            CRT_CUDA(create(g->streams[k]));
             // the first launch of a kernel on a device loads its code (CUDA loads modules lazily; a cold process spent ~0.2 s of
             // its first 4K frame on the second GPU doing that while the first one waited for the shared host thread): one work
             // item through the whole pipeline now, on every device, so that the first run_view starts warm
@@ -782,33 +767,33 @@ int crt_group_create(crt_scene* s, uint32_t width, uint32_t height, const int* d
             warm.range_set = true; warm.work_begin = 0; warm.work_end = 1;
             const float eye0[3] = {0, 0, 0}, M0[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
             crt_render_stats ws;
-            rc = wavefront_render(g->wf[k], g->scene_of(k), warm, eye0, M0, 1.0f, g->streams[k], &ws);
+            rc = wavefront_render(g->wf[k].get(), g->scene_of(k), warm, eye0, M0, 1.0f, g->streams[k].get(), &ws);
             if (rc != CRT_OK) return rc;
         }
         CRT_CUDA(cudaSetDevice(devices[0]));
-        CRT_CUDA(cudaMalloc(&g->d_linear, sizeof(float) * 3 * (size_t)width * height));
-        CRT_CUDA(cudaMalloc(&g->d_rgb8, 3 * (size_t)width * height));
-        CRT_CUDA(cudaEventCreate(&g->ev_r0));
-        CRT_CUDA(cudaEventCreate(&g->ev_r1));
-        for (cudaEvent_t& e : g->ev_band) CRT_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        CRT_CUDA(cudaStreamCreateWithFlags(&g->st_resolve, cudaStreamNonBlocking));
+        CRT_CUDA(g->d_linear.alloc(3 * (size_t)width * height));
+        CRT_CUDA(g->d_rgb8.alloc(3 * (size_t)width * height));
+        CRT_CUDA(create(g->ev_r0));
+        CRT_CUDA(create(g->ev_r1));
+        for (Event& e : g->ev_band) CRT_CUDA(create(e, cudaEventDisableTiming));
+        CRT_CUDA(create(g->st_resolve));
         if (n_devices > 1) {
             CRT_NCCL(g_nccl.CommInitAll(g->comms.data(), (int)n_devices, devices));
             // the first collective of a communicator sets up its connections (~0.2 s): spent here on the 24 bytes of pixel 0,
             // not inside the first frame (the buffers are cleared at the start of every run_view)
             for (uint32_t k = 0; k < n_devices; ++k) {
                 CRT_CUDA(cudaSetDevice(devices[k]));
-                CRT_CUDA(cudaMemsetAsync(wavefront_accum(g->wf[k]), 0, 3 * sizeof(long long), g->streams[k]));
+                CRT_CUDA(cudaMemsetAsync(wavefront_accum(g->wf[k].get()), 0, 3 * sizeof(long long), g->streams[k].get()));
             }
             CRT_NCCL(g_nccl.GroupStart());
             for (uint32_t k = 0; k < n_devices; ++k) {
-                long long* acc = wavefront_accum(g->wf[k]);
-                CRT_NCCL(g_nccl.Reduce(acc, acc, 3, ncclInt64, ncclSum, 0, g->comms[k], g->streams[k]));
+                long long* acc = wavefront_accum(g->wf[k].get());
+                CRT_NCCL(g_nccl.Reduce(acc, acc, 3, ncclInt64, ncclSum, 0, g->comms[k], g->streams[k].get()));
             }
             CRT_NCCL(g_nccl.GroupEnd());
             for (uint32_t k = 0; k < n_devices; ++k) {
                 CRT_CUDA(cudaSetDevice(devices[k]));
-                CRT_CUDA(cudaStreamSynchronize(g->streams[k]));
+                CRT_CUDA(cudaStreamSynchronize(g->streams[k].get()));
             }
             CRT_CUDA(cudaSetDevice(devices[0]));
         }
@@ -842,7 +827,7 @@ int crt_group_run_view(crt_group* g, const float eye[3], const float inv_view[9]
         if (g->rs.spp >= G) { rs.work_begin = (k * g->rs.spp / G) * npix; rs.work_end = ((k + 1) * g->rs.spp / G) * npix; }
         else { rs.work_begin = k * total / G; rs.work_end = (k + 1) * total / G; }
         CRT_CUDA(cudaSetDevice(g->devices[k]));
-        int rc = wavefront_begin(g->wf[k], g->scene_of(k), rs, eye, inv_view, tan_half, g->streams[k]);
+        int rc = wavefront_begin(g->wf[k].get(), g->scene_of(k), rs, eye, inv_view, tan_half, g->streams[k].get());
         if (rc != CRT_OK) return rc;
     }
     // one host thread feeds every GPU: a step enqueues one wavefront iteration where the GPU is ready for it
@@ -853,7 +838,7 @@ int crt_group_run_view(crt_group* g, const float eye[3], const float inv_view[9]
             if (done[k]) continue;
             CRT_CUDA(cudaSetDevice(g->devices[k]));
             bool d = false, progressed = false;
-            int rc = wavefront_step(g->wf[k], false, &d, &progressed);
+            int rc = wavefront_step(g->wf[k].get(), false, &d, &progressed);
             if (rc != CRT_OK) return rc;
             any = any || progressed;
             if (d) { done[k] = 1; --left; }
@@ -862,7 +847,7 @@ int crt_group_run_view(crt_group* g, const float eye[3], const float inv_view[9]
     }
     for (size_t k = 0; k < G; ++k) {
         CRT_CUDA(cudaSetDevice(g->devices[k]));
-        int rc = wavefront_finish(g->wf[k], &g->stats[k]);
+        int rc = wavefront_finish(g->wf[k].get(), &g->stats[k]);
         if (rc != CRT_OK) return rc;
     }
     // The collective: sum of the int64 buffers onto devices[0] (integer addition: the same buffer for every G), issued in bands
@@ -874,31 +859,31 @@ int crt_group_run_view(crt_group* g, const float eye[3], const float inv_view[9]
         // a band is at least 2^20 pixels (25 MB): a collective costs ~20 us before it moves a byte, the 800x600 frames go in one piece
         const unsigned long long band_px = std::max<unsigned long long>((npix + kGroupBands - 1) / kGroupBands, 1ull << 20);
         CRT_CUDA(cudaSetDevice(g->devices[0]));
-        CRT_CUDA(cudaEventRecord(g->ev_r0, g->streams[0]));
+        CRT_CUDA(cudaEventRecord(g->ev_r0.get(), g->streams[0].get()));
         int band = 0;
         for (unsigned long long px0 = 0; px0 < npix; px0 += band_px, ++band) {
             const unsigned long long cnt_px = std::min(band_px, npix - px0);
             CRT_NCCL(g_nccl.GroupStart());
             for (size_t k = 0; k < G; ++k) {
-                long long* acc = wavefront_accum(g->wf[k]) + 3 * px0;
-                CRT_NCCL(g_nccl.Reduce(acc, acc, (size_t)(3 * cnt_px), ncclInt64, ncclSum, 0, g->comms[k], g->streams[k]));
+                long long* acc = wavefront_accum(g->wf[k].get()) + 3 * px0;
+                CRT_NCCL(g_nccl.Reduce(acc, acc, (size_t)(3 * cnt_px), ncclInt64, ncclSum, 0, g->comms[k], g->streams[k].get()));
             }
             CRT_NCCL(g_nccl.GroupEnd());
             CRT_CUDA(cudaSetDevice(g->devices[0]));
-            CRT_CUDA(cudaEventRecord(g->ev_band[band % kGroupBands], g->streams[0]));
-            CRT_CUDA(cudaStreamWaitEvent(g->st_resolve, g->ev_band[band % kGroupBands], 0));
-            int rc = resolve_device(wavefront_accum(g->wf[0]) + 3 * px0, (uint32_t)cnt_px, g->rs.spp, g->d_linear + 3 * px0, g->d_rgb8 + 3 * px0,
-                                    g->st_resolve);
+            CRT_CUDA(cudaEventRecord(g->ev_band[band % kGroupBands].get(), g->streams[0].get()));
+            CRT_CUDA(cudaStreamWaitEvent(g->st_resolve.get(), g->ev_band[band % kGroupBands].get(), 0));
+            int rc = resolve_device(wavefront_accum(g->wf[0].get()) + 3 * px0, (uint32_t)cnt_px, g->rs.spp, g->d_linear.get() + 3 * px0, g->d_rgb8.get() + 3 * px0,
+                                    g->st_resolve.get());
             if (rc != CRT_OK) return rc;
         }
-        CRT_CUDA(cudaEventRecord(g->ev_r1, g->streams[0]));
+        CRT_CUDA(cudaEventRecord(g->ev_r1.get(), g->streams[0].get()));
         for (size_t k = 0; k < G; ++k) {
             CRT_CUDA(cudaSetDevice(g->devices[k]));
-            CRT_CUDA(cudaStreamSynchronize(g->streams[k]));
+            CRT_CUDA(cudaStreamSynchronize(g->streams[k].get()));
         }
         CRT_CUDA(cudaSetDevice(g->devices[0]));
-        CRT_CUDA(cudaStreamSynchronize(g->st_resolve));
-        CRT_CUDA(cudaEventElapsedTime(&g->reduce_ms, g->ev_r0, g->ev_r1));
+        CRT_CUDA(cudaStreamSynchronize(g->st_resolve.get()));
+        CRT_CUDA(cudaEventElapsedTime(&g->reduce_ms, g->ev_r0.get(), g->ev_r1.get()));
         g->resolved = true;
     }
     g->rendered = true;
@@ -909,7 +894,7 @@ int crt_group_run_view(crt_group* g, const float eye[3], const float inv_view[9]
 int crt_group_get_accum_i64(crt_group* g, int64_t* out) {
     CHECK_ARG(g && out, "crt_group_get_accum_i64: null argument");
     CRT_CUDA(cudaSetDevice(g->devices[0]));
-    CRT_CUDA(cudaMemcpy(out, wavefront_accum(g->wf[0]), sizeof(int64_t) * 3 * (size_t)g->width * g->height, cudaMemcpyDeviceToHost));
+    CRT_CUDA(cudaMemcpy(out, wavefront_accum(g->wf[0].get()), sizeof(int64_t) * 3 * (size_t)g->width * g->height, cudaMemcpyDeviceToHost));
     return CRT_OK;
 }
 
@@ -918,11 +903,11 @@ int crt_group_get_rgb8(crt_group* g, uint8_t* out) {
     CRT_CUDA(cudaSetDevice(g->devices[0]));
     const uint32_t npix = g->width * g->height;
     if (!g->resolved) {                          // one GPU: no collective, resolved here
-        int rc = resolve_device(wavefront_accum(g->wf[0]), npix, g->rs.spp, g->d_linear, g->d_rgb8, g->streams[0]);
+        int rc = resolve_device(wavefront_accum(g->wf[0].get()), npix, g->rs.spp, g->d_linear.get(), g->d_rgb8.get(), g->streams[0].get());
         if (rc != CRT_OK) return rc;
     }
-    CRT_CUDA(cudaMemcpyAsync(out, g->d_rgb8, 3 * (size_t)npix, cudaMemcpyDeviceToHost, g->streams[0]));
-    CRT_CUDA(cudaStreamSynchronize(g->streams[0]));
+    CRT_CUDA(cudaMemcpyAsync(out, g->d_rgb8.get(), 3 * (size_t)npix, cudaMemcpyDeviceToHost, g->streams[0].get()));
+    CRT_CUDA(cudaStreamSynchronize(g->streams[0].get()));
     return CRT_OK;
 }
 

@@ -713,35 +713,14 @@ __global__ void k_wide_emit(WideBuildView v, uint32_t n_level, uint32_t level_st
 // ------------------------------------------------------------------------------------------
 // host driver
 // ------------------------------------------------------------------------------------------
-#define BUILD_CHECK(x)                                                                           \
-    do {                                                                                         \
-        cudaError_t e_ = (x);                                                                    \
-        if (e_ != cudaSuccess) { rc = cuda_fail(e_, #x); goto done; }                            \
-    } while (0)
-
 int build_bvh_device(DeviceScene& ds, const float* d_verts, const float4* d_face_shade, uint32_t n, uint32_t thresh_n,
                      int builder, cudaStream_t st, float* build_ms) {
-    int rc = CRT_OK;
     const bool wide = (builder & 1) != 0;               // bit 0: 8-wide node layout, bit 1: PLOC topology
     const bool ploc = (builder & 2) != 0;
     if (thresh_n < 1) thresh_n = 1;
     if (wide && thresh_n > 15) thresh_n = 15;            // 7-bit leaf offsets inside a wide node
-    uint4* wnodes = nullptr;
-    int *work0 = nullptr, *work1 = nullptr, *tmp_ref = nullptr, *tmp_cnt = nullptr;
-    uint32_t *cnt_int = nullptr, *cnt_tri = nullptr, *off_int = nullptr, *off_tri = nullptr, *order8 = nullptr, *d_tot2 = nullptr;
-    uint8_t* last8 = nullptr;
-    float4 *pc_lo[2] = {nullptr, nullptr}, *pc_hi[2] = {nullptr, nullptr}, *pn_lo = nullptr, *pn_hi = nullptr;
-    int *p_nn = nullptr, *p_cl = nullptr, *p_cr = nullptr;
-    uint32_t *p_lower = nullptr, *p_rank = nullptr, *p_order = nullptr;
     const uint32_t n_tiles = (n + kSortTile - 1) / kSortTile;
     const int nb = (int)((n + 255) / 256);
-    float4 *tlo = nullptr, *thi = nullptr, *blo = nullptr, *bhi = nullptr;
-    float* bounds = nullptr;
-    uint64_t *keys0 = nullptr, *keys1 = nullptr;
-    uint32_t *vals0 = nullptr, *vals1 = nullptr, *ghist = nullptr, *scratch = nullptr, *flags = nullptr, *keep = nullptr,
-             *rank = nullptr, *d_total = nullptr;
-    int *left = nullptr, *right = nullptr, *first = nullptr, *last = nullptr, *pnode = nullptr, *pleaf = nullptr;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     uint32_t n_kept = 0;
     const float init_bounds[6] = {FLT_MAX, FLT_MAX, FLT_MAX, -FLT_MAX, -FLT_MAX, -FLT_MAX};
 
@@ -751,97 +730,101 @@ int build_bvh_device(DeviceScene& ds, const float* d_verts, const float4* d_face
     ds.builder = builder;
     if (n == 0) { if (build_ms) *build_ms = 0; return CRT_OK; }
 
-    BUILD_CHECK(cudaEventCreate(&ev0));
-    BUILD_CHECK(cudaEventCreate(&ev1));
-    BUILD_CHECK(cudaMalloc(&tlo, sizeof(float4) * n));
-    BUILD_CHECK(cudaMalloc(&thi, sizeof(float4) * n));
-    BUILD_CHECK(cudaMalloc(&bounds, sizeof(float) * 6));
-    BUILD_CHECK(cudaMalloc(&keys0, sizeof(uint64_t) * n));
-    BUILD_CHECK(cudaMalloc(&keys1, sizeof(uint64_t) * n));
-    BUILD_CHECK(cudaMalloc(&vals0, sizeof(uint32_t) * n));
-    BUILD_CHECK(cudaMalloc(&vals1, sizeof(uint32_t) * n));
-    BUILD_CHECK(cudaMalloc(&ghist, sizeof(uint32_t) * 256 * (size_t)n_tiles));
-    BUILD_CHECK(cudaMalloc(&scratch, sizeof(uint32_t) * (std::max((256 * (size_t)n_tiles + kScanTile - 1) / kScanTile,
-                                                             ((size_t)n + kScanTile - 1) / kScanTile) + 1)));
-    BUILD_CHECK(cudaMalloc(&d_total, sizeof(uint32_t)));
-    BUILD_CHECK(cudaMalloc(&ds.order, sizeof(uint32_t) * n));
-    BUILD_CHECK(cudaMalloc(&ds.last, n));
-    BUILD_CHECK(cudaMalloc(&ds.tri_geom, sizeof(float4) * 3 * (size_t)n));
-    BUILD_CHECK(cudaMalloc(&ds.tri_shade, sizeof(float4) * (size_t)n));
-    BUILD_CHECK(cudaMemsetAsync(ds.last, 0, n, st));
-    BUILD_CHECK(cudaMemcpyAsync(bounds, init_bounds, sizeof(init_bounds), cudaMemcpyHostToDevice, st));
+    // every temporary lives until the build has finished
+    Event ev0, ev1;
+    DevBuf<float4> tlo, thi, blo, bhi, pc_lo[2], pc_hi[2], pn_lo, pn_hi;
+    DevBuf<float> bounds;
+    DevBuf<uint64_t> keys0, keys1;
+    DevBuf<uint32_t> vals0, vals1, ghist, scratch, flags, keep, rank, d_total, p_lower, p_rank, p_order;
+    DevBuf<int> left, right, first, last, pnode, pleaf, p_nn, p_cl, p_cr;
+    DevBuf<uint4> wnodes;
+    DevBuf<int> work0, work1, tmp_ref, tmp_cnt;
+    DevBuf<uint32_t> cnt_int, cnt_tri, off_int, off_tri, order8, d_tot2;
+    DevBuf<uint8_t> last8;
+    CRT_CUDA(create(ev0));
+    CRT_CUDA(create(ev1));
+    CRT_CUDA(tlo.alloc(n));
+    CRT_CUDA(thi.alloc(n));
+    CRT_CUDA(bounds.alloc(6));
+    CRT_CUDA(keys0.alloc(n));
+    CRT_CUDA(keys1.alloc(n));
+    CRT_CUDA(vals0.alloc(n));
+    CRT_CUDA(vals1.alloc(n));
+    CRT_CUDA(ghist.alloc(256 * (size_t)n_tiles));
+    CRT_CUDA(scratch.alloc(std::max((256 * (size_t)n_tiles + kScanTile - 1) / kScanTile, ((size_t)n + kScanTile - 1) / kScanTile) + 1));
+    CRT_CUDA(d_total.alloc(1));
+    CRT_CUDA(ds.order.alloc(n));
+    CRT_CUDA(ds.last.alloc(n));
+    CRT_CUDA(ds.tri_geom.alloc(3 * (size_t)n));
+    CRT_CUDA(ds.tri_shade.alloc(n));
+    CRT_CUDA(cudaMemsetAsync(ds.last.get(), 0, n, st));
+    CRT_CUDA(cudaMemcpyAsync(bounds.get(), init_bounds, sizeof(init_bounds), cudaMemcpyHostToDevice, st));
 
-    BUILD_CHECK(cudaEventRecord(ev0, st));
-    k_tri_bounds<<<nb, 256, 0, st>>>(d_verts, n, tlo, thi, bounds);
-    k_morton<<<nb, 256, 0, st>>>(tlo, thi, n, bounds, keys0, vals0);
+    CRT_CUDA(cudaEventRecord(ev0.get(), st));
+    k_tri_bounds<<<nb, 256, 0, st>>>(d_verts, n, tlo.get(), thi.get(), bounds.get());
+    k_morton<<<nb, 256, 0, st>>>(tlo.get(), thi.get(), n, bounds.get(), keys0.get(), vals0.get());
     {
-        uint64_t *kin = keys0, *kout = keys1;
-        uint32_t *vin = vals0, *vout = vals1;
-        for (int pass = 0; pass < 8; ++pass) {
-            int shift = pass * 8;
-            k_sort_hist<<<n_tiles, 256, 0, st>>>(kin, n, shift, ghist, n_tiles);
-            BUILD_CHECK(exclusive_scan_u32(ghist, ghist, 256 * n_tiles, scratch, nullptr, st));
-            k_sort_scatter<<<n_tiles, 256, 0, st>>>(kin, vin, kout, vout, n, shift, ghist, n_tiles);
-            std::swap(kin, kout);
-            std::swap(vin, vout);
-        }
-        // 8 passes: result is back in keys0 / vals0
-        BUILD_CHECK(cudaMemcpyAsync(ds.order, vals0, sizeof(uint32_t) * n, cudaMemcpyDeviceToDevice, st));
+        uint64_t* sorted_keys = nullptr;                 // 8 passes: keys0 / vals0 again
+        uint32_t* sorted_vals = nullptr;
+        CRT_CUDA(radix_sort_pairs(keys0.get(), keys1.get(), vals0.get(), vals1.get(), n, 8, ghist.get(), scratch.get(), st, &sorted_keys,
+                                  &sorted_vals));
+        CRT_CUDA(cudaMemcpyAsync(ds.order.get(), sorted_vals, sizeof(uint32_t) * n, cudaMemcpyDeviceToDevice, st));
     }
-    BUILD_CHECK(cudaGetLastError());
+    CRT_CUDA(cudaGetLastError());
 
     if (n <= thresh_n) {
         n_kept = 1;
         if (!wide) {
-            BUILD_CHECK(cudaMalloc(&ds.nodes, sizeof(float4) * 4));
-            k_emit_single_leaf<<<1, 1, 0, st>>>((int)n, bounds, ds.nodes, ds.last);
+            CRT_CUDA(ds.nodes.alloc(4));
+            k_emit_single_leaf<<<1, 1, 0, st>>>((int)n, bounds.get(), ds.nodes.get(), ds.last.get());
         }
     } else {
         const uint32_t ni = n - 1;
         const int nbi = (int)((ni + 255) / 256);
-        BUILD_CHECK(cudaMalloc(&left, sizeof(int) * ni));
-        BUILD_CHECK(cudaMalloc(&right, sizeof(int) * ni));
-        BUILD_CHECK(cudaMalloc(&first, sizeof(int) * ni));
-        BUILD_CHECK(cudaMalloc(&last, sizeof(int) * ni));
-        BUILD_CHECK(cudaMalloc(&pnode, sizeof(int) * ni));
-        BUILD_CHECK(cudaMalloc(&pleaf, sizeof(int) * n));
-        BUILD_CHECK(cudaMalloc(&blo, sizeof(float4) * ni));
-        BUILD_CHECK(cudaMalloc(&bhi, sizeof(float4) * ni));
-        BUILD_CHECK(cudaMalloc(&flags, sizeof(uint32_t) * ni));
-        BUILD_CHECK(cudaMalloc(&keep, sizeof(uint32_t) * ni));
-        BUILD_CHECK(cudaMalloc(&rank, sizeof(uint32_t) * ni));
+        CRT_CUDA(left.alloc(ni));
+        CRT_CUDA(right.alloc(ni));
+        CRT_CUDA(first.alloc(ni));
+        CRT_CUDA(last.alloc(ni));
+        CRT_CUDA(pnode.alloc(ni));
+        CRT_CUDA(pleaf.alloc(n));
+        CRT_CUDA(blo.alloc(ni));
+        CRT_CUDA(bhi.alloc(ni));
+        CRT_CUDA(flags.alloc(ni));
+        CRT_CUDA(keep.alloc(ni));
+        CRT_CUDA(rank.alloc(ni));
         if (!ploc) {
-            BUILD_CHECK(cudaMemsetAsync(flags, 0, sizeof(uint32_t) * ni, st));
-            k_radix_tree<<<nbi, 256, 0, st>>>(keys0, (int)n, left, right, first, last, pnode, pleaf);
-            k_refit<<<nb, 256, 0, st>>>((int)n, ds.order, tlo, thi, left, right, pnode, pleaf, blo, bhi, flags);
+            CRT_CUDA(cudaMemsetAsync(flags.get(), 0, sizeof(uint32_t) * ni, st));
+            k_radix_tree<<<nbi, 256, 0, st>>>(keys0.get(), (int)n, left.get(), right.get(), first.get(), last.get(), pnode.get(), pleaf.get());
+            k_refit<<<nb, 256, 0, st>>>((int)n, ds.order.get(), tlo.get(), thi.get(), left.get(), right.get(), pnode.get(), pleaf.get(), blo.get(),
+                                        bhi.get(), flags.get());
         } else {
             for (int b = 0; b < 2; ++b) {
-                BUILD_CHECK(cudaMalloc(&pc_lo[b], sizeof(float4) * n));
-                BUILD_CHECK(cudaMalloc(&pc_hi[b], sizeof(float4) * n));
+                CRT_CUDA(pc_lo[b].alloc(n));
+                CRT_CUDA(pc_hi[b].alloc(n));
             }
-            BUILD_CHECK(cudaMalloc(&pn_lo, sizeof(float4) * ni));
-            BUILD_CHECK(cudaMalloc(&pn_hi, sizeof(float4) * ni));
-            BUILD_CHECK(cudaMalloc(&p_nn, sizeof(int) * n));
-            BUILD_CHECK(cudaMalloc(&p_cl, sizeof(int) * ni));
-            BUILD_CHECK(cudaMalloc(&p_cr, sizeof(int) * ni));
-            BUILD_CHECK(cudaMalloc(&p_lower, sizeof(uint32_t) * n));
-            BUILD_CHECK(cudaMalloc(&p_rank, sizeof(uint32_t) * n));
-            BUILD_CHECK(cudaMalloc(&p_order, sizeof(uint32_t) * n));
-            k_ploc_init<<<nb, 256, 0, st>>>(n, ds.order, tlo, thi, pc_lo[0], pc_hi[0]);
+            CRT_CUDA(pn_lo.alloc(ni));
+            CRT_CUDA(pn_hi.alloc(ni));
+            CRT_CUDA(p_nn.alloc(n));
+            CRT_CUDA(p_cl.alloc(ni));
+            CRT_CUDA(p_cr.alloc(ni));
+            CRT_CUDA(p_lower.alloc(n));
+            CRT_CUDA(p_rank.alloc(n));
+            CRT_CUDA(p_order.alloc(n));
+            k_ploc_init<<<nb, 256, 0, st>>>(n, ds.order.get(), tlo.get(), thi.get(), pc_lo[0].get(), pc_hi[0].get());
             std::vector<uint32_t> round_start;            // creation index at which every round begins
             uint32_t m = n, created = 0;
             int cur = 0;
             while (m > 1) {
                 const int nbm = (int)((m + 255) / 256);
-                k_ploc_nn<<<nbm, 256, 0, st>>>((int)m, pc_lo[cur], pc_hi[cur], p_nn);
-                k_ploc_lower<<<nbm, 256, 0, st>>>((int)m, p_nn, p_lower);
-                BUILD_CHECK(exclusive_scan_u32(p_lower, p_rank, m, scratch, d_total, st));
-                k_ploc_merge<<<nbm, 256, 0, st>>>((int)m, created, pc_lo[cur], pc_hi[cur], p_nn, p_rank, pc_lo[cur ^ 1], pc_hi[cur ^ 1],
-                                                  p_cl, p_cr, pn_lo, pn_hi);
+                k_ploc_nn<<<nbm, 256, 0, st>>>((int)m, pc_lo[cur].get(), pc_hi[cur].get(), p_nn.get());
+                k_ploc_lower<<<nbm, 256, 0, st>>>((int)m, p_nn.get(), p_lower.get());
+                CRT_CUDA(exclusive_scan_u32(p_lower.get(), p_rank.get(), m, scratch.get(), d_total.get(), st));
+                k_ploc_merge<<<nbm, 256, 0, st>>>((int)m, created, pc_lo[cur].get(), pc_hi[cur].get(), p_nn.get(), p_rank.get(), pc_lo[cur ^ 1].get(),
+                                                  pc_hi[cur ^ 1].get(), p_cl.get(), p_cr.get(), pn_lo.get(), pn_hi.get());
                 uint32_t merged = 0;
-                BUILD_CHECK(cudaMemcpyAsync(&merged, d_total, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-                BUILD_CHECK(cudaStreamSynchronize(st));
-                if (merged == 0 || merged > m / 2) { set_error("PLOC: a round merged nothing"); rc = CRT_ERR_STATE; goto done; }
+                CRT_CUDA(cudaMemcpyAsync(&merged, d_total.get(), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+                CRT_CUDA(cudaStreamSynchronize(st));
+                if (merged == 0 || merged > m / 2) { set_error("PLOC: a round merged nothing"); return CRT_ERR_STATE; }
                 round_start.push_back(created);
                 // Every round adds at most one level, so the number of rounds bounds the depth of the tree. The pair-node
                 // traversal pushes onto a stack of kStackSize entries without a bounds check (a Karras tree cannot be deeper
@@ -850,102 +833,90 @@ int build_bvh_device(DeviceScene& ds, const float* d_verts, const float4* d_face
                 if (round_start.size() >= (size_t)(wide ? 1024 : kStackSize - 1)) {
                     set_error("PLOC: the agglomeration needs more rounds than the traversal stack is deep (" + std::to_string(round_start.size()) +
                               "); build this scene with CRT_BUILDER_LBVH / CRT_BUILDER_LBVH8");
-                    rc = CRT_ERR_STATE;
-                    goto done;
+                    return CRT_ERR_STATE;
                 }
                 created += merged;
                 m -= merged;
                 cur ^= 1;
             }
-            if (created != ni) { set_error("PLOC: merge count mismatch"); rc = CRT_ERR_STATE; goto done; }
+            if (created != ni) { set_error("PLOC: merge count mismatch"); return CRT_ERR_STATE; }
             round_start.push_back(created);
-            k_ploc_root<<<1, 1, 0, st>>>((int)n, first, last);
+            k_ploc_root<<<1, 1, 0, st>>>((int)n, first.get(), last.get());
             for (size_t r = round_start.size() - 1; r-- > 0;) {
                 const uint32_t c0 = round_start[r], c1 = round_start[r + 1];
-                k_ploc_finalize<<<(int)((c1 - c0 + 255) / 256), 256, 0, st>>>(c0, c1, (int)ni, p_cl, p_cr, pn_lo, pn_hi, ds.order, left, right,
-                                                                               first, last, blo, bhi, p_order);
+                k_ploc_finalize<<<(int)((c1 - c0 + 255) / 256), 256, 0, st>>>(c0, c1, (int)ni, p_cl.get(), p_cr.get(), pn_lo.get(), pn_hi.get(),
+                                                                               ds.order.get(), left.get(), right.get(), first.get(), last.get(),
+                                                                               blo.get(), bhi.get(), p_order.get());
             }
             std::swap(ds.order, p_order);                 // depth-first order replaces the Morton order
         }
-        k_keep_flags<<<nbi, 256, 0, st>>>((int)ni, first, last, thresh_n, keep);
-        BUILD_CHECK(exclusive_scan_u32(keep, rank, ni, scratch, d_total, st));
-        BUILD_CHECK(cudaMemcpyAsync(&n_kept, d_total, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        BUILD_CHECK(cudaStreamSynchronize(st));
+        k_keep_flags<<<nbi, 256, 0, st>>>((int)ni, first.get(), last.get(), thresh_n, keep.get());
+        CRT_CUDA(exclusive_scan_u32(keep.get(), rank.get(), ni, scratch.get(), d_total.get(), st));
+        CRT_CUDA(cudaMemcpyAsync(&n_kept, d_total.get(), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        CRT_CUDA(cudaStreamSynchronize(st));
         if (!wide) {
-            BUILD_CHECK(cudaMalloc(&ds.nodes, sizeof(float4) * 4 * (size_t)n_kept));
-            k_emit_nodes<<<nbi, 256, 0, st>>>((int)ni, keep, rank, left, right, first, last, ds.order, tlo, thi, blo, bhi, ds.nodes,
-                                              ds.last);
+            CRT_CUDA(ds.nodes.alloc(4 * (size_t)n_kept));
+            k_emit_nodes<<<nbi, 256, 0, st>>>((int)ni, keep.get(), rank.get(), left.get(), right.get(), first.get(), last.get(), ds.order.get(),
+                                              tlo.get(), thi.get(), blo.get(), bhi.get(), ds.nodes.get(), ds.last.get());
         }
     }
     if (wide) {
         // breadth-first collapse into 80-byte nodes; at most one wide node per expandable radix node
         const size_t cap = std::max<uint32_t>(n_kept, 1);
-        BUILD_CHECK(cudaMalloc(&wnodes, sizeof(uint4) * 5 * cap));
-        BUILD_CHECK(cudaMalloc(&work0, sizeof(int) * cap));
-        BUILD_CHECK(cudaMalloc(&work1, sizeof(int) * cap));
-        BUILD_CHECK(cudaMalloc(&tmp_ref, sizeof(int) * 8 * cap));
-        BUILD_CHECK(cudaMalloc(&tmp_cnt, sizeof(int) * 8 * cap));
-        BUILD_CHECK(cudaMalloc(&cnt_int, sizeof(uint32_t) * cap));
-        BUILD_CHECK(cudaMalloc(&cnt_tri, sizeof(uint32_t) * cap));
-        BUILD_CHECK(cudaMalloc(&off_int, sizeof(uint32_t) * cap));
-        BUILD_CHECK(cudaMalloc(&off_tri, sizeof(uint32_t) * cap));
-        BUILD_CHECK(cudaMalloc(&d_tot2, sizeof(uint32_t) * 2));
-        BUILD_CHECK(cudaMalloc(&order8, sizeof(uint32_t) * n));
-        BUILD_CHECK(cudaMalloc(&last8, n));
-        BUILD_CHECK(cudaMemsetAsync(last8, 0, n, st));
+        CRT_CUDA(wnodes.alloc(5 * cap));
+        CRT_CUDA(work0.alloc(cap));
+        CRT_CUDA(work1.alloc(cap));
+        CRT_CUDA(tmp_ref.alloc(8 * cap));
+        CRT_CUDA(tmp_cnt.alloc(8 * cap));
+        CRT_CUDA(cnt_int.alloc(cap));
+        CRT_CUDA(cnt_tri.alloc(cap));
+        CRT_CUDA(off_int.alloc(cap));
+        CRT_CUDA(off_tri.alloc(cap));
+        CRT_CUDA(d_tot2.alloc(2));
+        CRT_CUDA(order8.alloc(n));
+        CRT_CUDA(last8.alloc(n));
+        CRT_CUDA(cudaMemsetAsync(last8.get(), 0, n, st));
         WideBuildView v;
-        v.left = left; v.right = right; v.first = first; v.last = last; v.blo = blo; v.bhi = bhi; v.tlo = tlo; v.thi = thi;
-        v.order = ds.order; v.scene_bounds = bounds; v.n_tris = (int)n; v.thresh = thresh_n;
+        v.left = left.get(); v.right = right.get(); v.first = first.get(); v.last = last.get(); v.blo = blo.get(); v.bhi = bhi.get();
+        v.tlo = tlo.get(); v.thi = thi.get(); v.order = ds.order.get(); v.scene_bounds = bounds.get(); v.n_tris = (int)n; v.thresh = thresh_n;
         const int root = n <= thresh_n ? -1 : 0;
-        BUILD_CHECK(cudaMemcpyAsync(work0, &root, sizeof(int), cudaMemcpyHostToDevice, st));
+        CRT_CUDA(cudaMemcpyAsync(work0.get(), &root, sizeof(int), cudaMemcpyHostToDevice, st));
         uint32_t level_start = 0, n_level = 1, tri_cursor = 0, levels = 0;
-        int *wcur = work0, *wnext = work1;
+        int *wcur = work0.get(), *wnext = work1.get();
         while (n_level > 0) {
             // the traversal stack holds one entry per level (crt_wide.cuh kWideStack)
-            if (++levels > (uint32_t)kWideStack) { set_error("wide BVH: tree deeper than the traversal stack"); rc = CRT_ERR_STATE; goto done; }
-            if ((size_t)level_start + n_level > cap) { set_error("wide BVH: node bound exceeded"); rc = CRT_ERR_STATE; goto done; }
+            if (++levels > (uint32_t)kWideStack) { set_error("wide BVH: tree deeper than the traversal stack"); return CRT_ERR_STATE; }
+            if ((size_t)level_start + n_level > cap) { set_error("wide BVH: node bound exceeded"); return CRT_ERR_STATE; }
             const int nbl = (int)((n_level + 127) / 128);
-            k_wide_collapse<<<nbl, 128, 0, st>>>(v, n_level, wcur, tmp_ref, tmp_cnt, cnt_int, cnt_tri);
-            BUILD_CHECK(exclusive_scan_u32(cnt_int, off_int, n_level, scratch, d_tot2, st));
-            BUILD_CHECK(exclusive_scan_u32(cnt_tri, off_tri, n_level, scratch, d_tot2 + 1, st));
+            k_wide_collapse<<<nbl, 128, 0, st>>>(v, n_level, wcur, tmp_ref.get(), tmp_cnt.get(), cnt_int.get(), cnt_tri.get());
+            CRT_CUDA(exclusive_scan_u32(cnt_int.get(), off_int.get(), n_level, scratch.get(), d_tot2.get(), st));
+            CRT_CUDA(exclusive_scan_u32(cnt_tri.get(), off_tri.get(), n_level, scratch.get(), d_tot2.get() + 1, st));
             uint32_t tot[2] = {0, 0};
-            BUILD_CHECK(cudaMemcpyAsync(tot, d_tot2, sizeof(tot), cudaMemcpyDeviceToHost, st));
-            BUILD_CHECK(cudaStreamSynchronize(st));
-            k_wide_emit<<<nbl, 128, 0, st>>>(v, n_level, level_start, level_start + n_level, tri_cursor, wcur, tmp_ref, tmp_cnt, off_int,
-                                             off_tri, wnodes, wnext, order8, last8);
-            BUILD_CHECK(cudaGetLastError());
+            CRT_CUDA(cudaMemcpyAsync(tot, d_tot2.get(), sizeof(tot), cudaMemcpyDeviceToHost, st));
+            CRT_CUDA(cudaStreamSynchronize(st));
+            k_wide_emit<<<nbl, 128, 0, st>>>(v, n_level, level_start, level_start + n_level, tri_cursor, wcur, tmp_ref.get(), tmp_cnt.get(),
+                                             off_int.get(), off_tri.get(), wnodes.get(), wnext, order8.get(), last8.get());
+            CRT_CUDA(cudaGetLastError());
             level_start += n_level;
             n_level = tot[0];
             tri_cursor += tot[1];
             std::swap(wcur, wnext);
         }
-        if (tri_cursor != n) { set_error("wide BVH: triangle count mismatch"); rc = CRT_ERR_STATE; goto done; }
+        if (tri_cursor != n) { set_error("wide BVH: triangle count mismatch"); return CRT_ERR_STATE; }
         n_kept = level_start;
-        BUILD_CHECK(cudaMalloc(&ds.nodes, sizeof(uint4) * 5 * (size_t)n_kept));
-        BUILD_CHECK(cudaMemcpyAsync(ds.nodes, wnodes, sizeof(uint4) * 5 * (size_t)n_kept, cudaMemcpyDeviceToDevice, st));
+        CRT_CUDA(ds.nodes.alloc(5 * (size_t)n_kept));
+        CRT_CUDA(cudaMemcpyAsync(ds.nodes.get(), wnodes.get(), sizeof(uint4) * 5 * (size_t)n_kept, cudaMemcpyDeviceToDevice, st));
         std::swap(ds.order, order8);
         std::swap(ds.last, last8);
     }
-    k_emit_tris<<<nb, 256, 0, st>>>(n, ds.order, ds.last, d_verts, d_face_shade, ds.tri_geom, ds.tri_shade);
-    BUILD_CHECK(cudaGetLastError());
-    BUILD_CHECK(cudaEventRecord(ev1, st));
-    BUILD_CHECK(cudaStreamSynchronize(st));
-    BUILD_CHECK(cudaMemcpy(ds.bounds, bounds, sizeof(float) * 6, cudaMemcpyDeviceToHost));
+    k_emit_tris<<<nb, 256, 0, st>>>(n, ds.order.get(), ds.last.get(), d_verts, d_face_shade, ds.tri_geom.get(), ds.tri_shade.get());
+    CRT_CUDA(cudaGetLastError());
+    CRT_CUDA(cudaEventRecord(ev1.get(), st));
+    CRT_CUDA(cudaStreamSynchronize(st));
+    CRT_CUDA(cudaMemcpy(ds.bounds, bounds.get(), sizeof(float) * 6, cudaMemcpyDeviceToHost));
     ds.n_nodes = n_kept;
-    if (build_ms) BUILD_CHECK(cudaEventElapsedTime(build_ms, ev0, ev1));
-
-done:
-    cudaFree(tlo); cudaFree(thi); cudaFree(blo); cudaFree(bhi); cudaFree(bounds);
-    cudaFree(keys0); cudaFree(keys1); cudaFree(vals0); cudaFree(vals1); cudaFree(ghist); cudaFree(scratch);
-    cudaFree(flags); cudaFree(keep); cudaFree(rank); cudaFree(d_total);
-    cudaFree(left); cudaFree(right); cudaFree(first); cudaFree(last); cudaFree(pnode); cudaFree(pleaf);
-    cudaFree(wnodes); cudaFree(work0); cudaFree(work1); cudaFree(tmp_ref); cudaFree(tmp_cnt); cudaFree(cnt_int); cudaFree(cnt_tri);
-    cudaFree(off_int); cudaFree(off_tri); cudaFree(order8); cudaFree(last8); cudaFree(d_tot2);
-    for (int b = 0; b < 2; ++b) { cudaFree(pc_lo[b]); cudaFree(pc_hi[b]); }
-    cudaFree(pn_lo); cudaFree(pn_hi); cudaFree(p_nn); cudaFree(p_cl); cudaFree(p_cr); cudaFree(p_lower); cudaFree(p_rank); cudaFree(p_order);
-    if (ev0) cudaEventDestroy(ev0);
-    if (ev1) cudaEventDestroy(ev1);
-    return rc;
+    if (build_ms) CRT_CUDA(cudaEventElapsedTime(build_ms, ev0.get(), ev1.get()));
+    return CRT_OK;
 }
 
 }  // namespace crt

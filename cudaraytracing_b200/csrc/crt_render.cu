@@ -31,39 +31,20 @@ namespace crt {
 // =============================================================================================
 // scene upload
 // =============================================================================================
-void DeviceScene::release() {
-    cudaFree(nodes); cudaFree(tri_geom); cudaFree(tri_shade); cudaFree(order); cudaFree(last);
-    cudaFree(mats); cudaFree(light_tris); cudaFree(lights); cudaFree(light_cdf);
-    light_cdf = nullptr;
-    nodes = tri_geom = tri_shade = mats = light_tris = nullptr;
-    order = nullptr; last = nullptr; lights = nullptr;
-    n_tris = n_nodes = n_mats = n_lights = n_light_tris = 0;
-}
-
 int clone_scene(const DeviceScene& src, int device, DeviceScene& dst) {
     CRT_CUDA(cudaSetDevice(device));
-    dst.release();
-    dst = src;                                                  // counts, flags, bounds; the pointers are replaced below
+    dst = DeviceScene();
+    static_cast<SceneInfo&>(dst) = src;                         // counts, flags, bounds
     dst.device = device;
-    dst.nodes = dst.tri_geom = dst.tri_shade = dst.mats = dst.light_tris = nullptr;
-    dst.order = nullptr; dst.last = nullptr; dst.lights = nullptr; dst.light_cdf = nullptr;
-    auto copy = [&](auto*& d, const auto* s_ptr, size_t bytes) -> int {
-        if (!s_ptr || bytes == 0) return CRT_OK;
-        CRT_CUDA(cudaMalloc((void**)&d, bytes));
-        CRT_CUDA(cudaMemcpyPeer(d, device, s_ptr, src.device, bytes));
-        return CRT_OK;
-    };
-    int rc = CRT_OK;
-    const size_t node_bytes = sizeof(float4) * (src.wide ? 5 : 4) * (size_t)src.n_nodes;
-    if ((rc = copy(dst.nodes, src.nodes, node_bytes)) != CRT_OK) return rc;
-    if ((rc = copy(dst.tri_geom, src.tri_geom, sizeof(float4) * 3 * (size_t)src.n_tris)) != CRT_OK) return rc;
-    if ((rc = copy(dst.tri_shade, src.tri_shade, sizeof(float4) * (size_t)src.n_tris)) != CRT_OK) return rc;
-    if ((rc = copy(dst.order, src.order, sizeof(uint32_t) * (size_t)src.n_tris)) != CRT_OK) return rc;
-    if ((rc = copy(dst.last, src.last, (size_t)src.n_tris)) != CRT_OK) return rc;
-    if ((rc = copy(dst.mats, src.mats, sizeof(float4) * 5 * (size_t)src.n_mats)) != CRT_OK) return rc;
-    if ((rc = copy(dst.light_tris, src.light_tris, sizeof(float4) * 4 * (size_t)src.n_light_tris)) != CRT_OK) return rc;
-    if ((rc = copy(dst.lights, src.lights, sizeof(int4) * (size_t)src.n_lights)) != CRT_OK) return rc;
-    if ((rc = copy(dst.light_cdf, src.light_cdf, sizeof(float) * (size_t)src.n_light_tris)) != CRT_OK) return rc;
+    cudaError_t e = cudaSuccess;
+    DeviceScene::for_each_table([&](auto table) {
+        const auto& s = src.*table;
+        auto& d = dst.*table;
+        if (e != cudaSuccess || s.size() == 0) return;
+        e = d.alloc(s.size());
+        if (e == cudaSuccess) e = cudaMemcpyPeer(d.get(), device, s.get(), src.device, sizeof(*s.get()) * s.size());
+    });
+    CRT_CUDA(e);
     CRT_CUDA(cudaDeviceSynchronize());
     return CRT_OK;
 }
@@ -77,7 +58,7 @@ static uint32_t env_u32(const char* name, uint32_t dflt) {
 
 int upload_scene(const HostScene& hs, uint32_t thresh_n, int builder, int device, DeviceScene& ds, float* build_ms) {
     CRT_CUDA(cudaSetDevice(device));
-    ds.release();
+    ds = DeviceScene();
     ds.device = device;
     const size_t n = hs.n_tris();
     if (n > 0x7fffffffu / 4) { set_error("scene too large (more than 2^29 triangles)"); return CRT_ERR_INVALID; }
@@ -120,36 +101,31 @@ int upload_scene(const HostScene& hs, uint32_t thresh_n, int builder, int device
     ds.n_lights = (uint32_t)lights.size();
     ds.n_light_tris = (uint32_t)(ltris.size() / 4);
     if (!mats.empty()) {
-        CRT_CUDA(cudaMalloc(&ds.mats, sizeof(float4) * mats.size()));
-        CRT_CUDA(cudaMemcpy(ds.mats, mats.data(), sizeof(float4) * mats.size(), cudaMemcpyHostToDevice));
+        CRT_CUDA(ds.mats.alloc(mats.size()));
+        CRT_CUDA(cudaMemcpy(ds.mats.get(), mats.data(), sizeof(float4) * mats.size(), cudaMemcpyHostToDevice));
     }
     if (!lights.empty()) {
-        CRT_CUDA(cudaMalloc(&ds.lights, sizeof(int4) * lights.size()));
-        CRT_CUDA(cudaMemcpy(ds.lights, lights.data(), sizeof(int4) * lights.size(), cudaMemcpyHostToDevice));
-        CRT_CUDA(cudaMalloc(&ds.light_tris, sizeof(float4) * ltris.size()));
-        CRT_CUDA(cudaMemcpy(ds.light_tris, ltris.data(), sizeof(float4) * ltris.size(), cudaMemcpyHostToDevice));
+        CRT_CUDA(ds.lights.alloc(lights.size()));
+        CRT_CUDA(cudaMemcpy(ds.lights.get(), lights.data(), sizeof(int4) * lights.size(), cudaMemcpyHostToDevice));
+        CRT_CUDA(ds.light_tris.alloc(ltris.size()));
+        CRT_CUDA(cudaMemcpy(ds.light_tris.get(), ltris.data(), sizeof(float4) * ltris.size(), cudaMemcpyHostToDevice));
         if (hs.light_cdf.size() != ltris.size() / 4) { set_error("light table out of date (finish_objects not called)"); return CRT_ERR_STATE; }
-        CRT_CUDA(cudaMalloc(&ds.light_cdf, sizeof(float) * hs.light_cdf.size()));
-        CRT_CUDA(cudaMemcpy(ds.light_cdf, hs.light_cdf.data(), sizeof(float) * hs.light_cdf.size(), cudaMemcpyHostToDevice));
+        CRT_CUDA(ds.light_cdf.alloc(hs.light_cdf.size()));
+        CRT_CUDA(cudaMemcpy(ds.light_cdf.get(), hs.light_cdf.data(), sizeof(float) * hs.light_cdf.size(), cudaMemcpyHostToDevice));
     }
     // geometry in face order for the builder
-    float* d_verts = nullptr;
-    float4* d_shade = nullptr;
-    int rc = CRT_OK;
+    DevBuf<float> d_verts;
+    DevBuf<float4> d_shade;
     if (n > 0) {
         std::vector<float4> shade(n);
         for (size_t t = 0; t < n; ++t)
             shade[t] = make_float4(hs.normal[3 * t], hs.normal[3 * t + 1], hs.normal[3 * t + 2], bits_f((uint32_t)hs.mat[t]));
-        CRT_CUDA(cudaMalloc(&d_verts, sizeof(float) * 9 * n));
-        cudaError_t e = cudaMalloc(&d_shade, sizeof(float4) * n);
-        if (e != cudaSuccess) { cudaFree(d_verts); return cuda_fail(e, "cudaMalloc face_shade"); }
-        cudaMemcpy(d_verts, hs.verts.data(), sizeof(float) * 9 * n, cudaMemcpyHostToDevice);
-        cudaMemcpy(d_shade, shade.data(), sizeof(float4) * n, cudaMemcpyHostToDevice);
+        CRT_CUDA(d_verts.alloc(9 * n));
+        CRT_CUDA(d_shade.alloc(n));
+        cudaMemcpy(d_verts.get(), hs.verts.data(), sizeof(float) * 9 * n, cudaMemcpyHostToDevice);
+        cudaMemcpy(d_shade.get(), shade.data(), sizeof(float4) * n, cudaMemcpyHostToDevice);
     }
-    rc = build_bvh_device(ds, d_verts, d_shade, (uint32_t)n, thresh_n, builder, 0, build_ms);
-    cudaFree(d_verts);
-    cudaFree(d_shade);
-    return rc;
+    return build_bvh_device(ds, d_verts.get(), d_shade.get(), (uint32_t)n, thresh_n, builder, 0, build_ms);
 }
 
 // =============================================================================================
@@ -162,6 +138,9 @@ CRT_DEV void trace_queue(const SceneView& sc, uint32_t n, uint32_t* fetch, Load 
     else if (WIDE) trace_persistent_queue<MODE, WideWalker>(sc, n, fetch, load, done);
     else trace_persistent_queue<MODE, PairWalker>(sc, n, fetch, load, done);
 }
+// with_layout(wide, f): f(std::true_type()) or f(std::false_type()), so that f can pass WIDE to a kernel as W.value
+template <typename F>
+static auto with_layout(bool wide, F&& f) { return wide ? f(std::true_type()) : f(std::false_type()); }
 template <int MODE, bool WIDE>
 CRT_DEV HitRec trace_one(const SceneView& sc, V3 o, V3 d, float tmax) {
     if (WIDE) return traverse_wide<MODE>(sc, o, d, tmax);
@@ -203,66 +182,45 @@ static int num_sms() {
 struct RayBatcher {
     int device = 0;
     int blocks = 0;
-    uint32_t* fetch = nullptr;                  // two queue counters, 128 bytes apart (one per pipeline slot)
+    DevBuf<uint32_t> fetch;                     // two queue counters, 128 bytes apart (one per pipeline slot)
     bool chunk_from_env = false;
-    cudaEvent_t ev_a[2] = {nullptr, nullptr}, ev_b[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr};
-    cudaStream_t st[2] = {nullptr, nullptr};
+    Event ev_a[2], ev_b[2], ev_done[2];
+    Stream st[2];
     // host-buffer path, allocated on first use
     uint64_t chunk = 0;                         // rays per chunk
-    float4* d_rays[2] = {nullptr, nullptr};
-    float* d_t[2] = {nullptr, nullptr};
-    int* d_face[2] = {nullptr, nullptr};
-    float4* h_rays[2] = {nullptr, nullptr};     // pinned staging for pageable callers
-    float* h_t[2] = {nullptr, nullptr};
-    int* h_face[2] = {nullptr, nullptr};
+    DevBuf<float4> d_rays[2];
+    DevBuf<float> d_t[2];
+    DevBuf<int> d_face[2];
+    Pinned<float4> h_rays[2];                   // pinned staging for pageable callers
+    Pinned<float> h_t[2];
+    Pinned<int> h_face[2];
     // CRT_RAY_SORTED, allocated on first use and grown: keys / permutation (ping-pong), the ordered copy of the rays and of the hits
     struct SortBufs {
         uint64_t cap = 0;
-        uint64_t *k0 = nullptr, *k1 = nullptr;
-        uint32_t *v0 = nullptr, *v1 = nullptr, *ghist = nullptr, *scratch = nullptr;
-        float4* rays = nullptr;
-        float* t = nullptr;
-        int* face = nullptr;
-        void release() {
-            cudaFree(k0); cudaFree(k1); cudaFree(v0); cudaFree(v1); cudaFree(ghist); cudaFree(scratch); cudaFree(rays); cudaFree(t); cudaFree(face);
-            *this = SortBufs();
-        }
+        DevBuf<uint64_t> k0, k1;
+        DevBuf<uint32_t> v0, v1, ghist, scratch;
+        DevBuf<float4> rays;
+        DevBuf<float> t;
+        DevBuf<int> face;
     } sort[2];
 };
+void StateDelete::operator()(RayBatcher* b) const { delete b; }
 
-int ray_batcher_create(const DeviceScene& ds, RayBatcher** out) {
-    RayBatcher* b = new RayBatcher();
+int ray_batcher_create(const DeviceScene& ds, RayBatcherPtr& out) {
+    RayBatcherPtr b(new RayBatcher());
     b->device = ds.device;
-    *out = b;                                                  // destroyed by the caller on failure, too
-    CRT_CUDA(cudaMalloc(&b->fetch, 256));
+    CRT_CUDA(b->fetch.alloc(64));
     for (int k = 0; k < 2; ++k) {
-        CRT_CUDA(cudaEventCreate(&b->ev_a[k]));
-        CRT_CUDA(cudaEventCreate(&b->ev_b[k]));
-        CRT_CUDA(cudaEventCreateWithFlags(&b->ev_done[k], cudaEventDisableTiming));
-        CRT_CUDA(cudaStreamCreateWithFlags(&b->st[k], cudaStreamNonBlocking));
+        CRT_CUDA(create(b->ev_a[k]));
+        CRT_CUDA(create(b->ev_b[k]));
+        CRT_CUDA(create(b->ev_done[k], cudaEventDisableTiming));
+        CRT_CUDA(create(b->st[k]));
     }
     int occ = 0;
-    if (ds.wide) CRT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_trace_batch<0, true>, 128, 0));
-    else CRT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_trace_batch<0, false>, 128, 0));
+    CRT_CUDA(with_layout(ds.wide, [&](auto W) { return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_trace_batch<0, W.value>, 128, 0); }));
     b->blocks = num_sms() * std::max(occ, 1);
+    out = std::move(b);
     return CRT_OK;
-}
-
-void ray_batcher_destroy(RayBatcher* b) {
-    if (!b) return;
-    cudaFree(b->fetch);
-    for (int k = 0; k < 2; ++k) {
-        if (b->ev_a[k]) cudaEventDestroy(b->ev_a[k]);
-        if (b->ev_b[k]) cudaEventDestroy(b->ev_b[k]);
-        if (b->ev_done[k]) cudaEventDestroy(b->ev_done[k]);
-        if (b->st[k]) cudaStreamDestroy(b->st[k]);
-        cudaFree(b->d_rays[k]); cudaFree(b->d_t[k]); cudaFree(b->d_face[k]);
-        if (b->h_rays[k]) cudaFreeHost(b->h_rays[k]);
-        if (b->h_t[k]) cudaFreeHost(b->h_t[k]);
-        if (b->h_face[k]) cudaFreeHost(b->h_face[k]);
-        b->sort[k].release();
-    }
-    delete b;
 }
 
 // ---- CRT_RAY_SORTED: "warp-coherent ray sorting" as an option of the batch calls --------------------------------------------------
@@ -309,17 +267,17 @@ __global__ void k_scatter_hits(const uint32_t* __restrict__ perm, uint32_t n, co
 }
 static int ensure_sort_bufs(RayBatcher::SortBufs& sb, uint64_t cnt) {
     if (sb.cap >= cnt) return CRT_OK;
-    sb.release();
+    sb = RayBatcher::SortBufs();
     const uint32_t n = (uint32_t)cnt;
-    CRT_CUDA(cudaMalloc(&sb.k0, sizeof(uint64_t) * cnt));
-    CRT_CUDA(cudaMalloc(&sb.k1, sizeof(uint64_t) * cnt));
-    CRT_CUDA(cudaMalloc(&sb.v0, sizeof(uint32_t) * cnt));
-    CRT_CUDA(cudaMalloc(&sb.v1, sizeof(uint32_t) * cnt));
-    CRT_CUDA(cudaMalloc(&sb.ghist, sizeof(uint32_t) * radix_sort_hist_words(n)));
-    CRT_CUDA(cudaMalloc(&sb.scratch, sizeof(uint32_t) * radix_sort_scratch_words(n)));
-    CRT_CUDA(cudaMalloc(&sb.rays, sizeof(float4) * 2 * cnt));
-    CRT_CUDA(cudaMalloc(&sb.t, sizeof(float) * cnt));
-    CRT_CUDA(cudaMalloc(&sb.face, sizeof(int) * cnt));
+    CRT_CUDA(sb.k0.alloc(cnt));
+    CRT_CUDA(sb.k1.alloc(cnt));
+    CRT_CUDA(sb.v0.alloc(cnt));
+    CRT_CUDA(sb.v1.alloc(cnt));
+    CRT_CUDA(sb.ghist.alloc(radix_sort_hist_words(n)));
+    CRT_CUDA(sb.scratch.alloc(radix_sort_scratch_words(n)));
+    CRT_CUDA(sb.rays.alloc(2 * cnt));
+    CRT_CUDA(sb.t.alloc(cnt));
+    CRT_CUDA(sb.face.alloc(cnt));
     sb.cap = cnt;
     return CRT_OK;
 }
@@ -327,13 +285,10 @@ static int ensure_sort_bufs(RayBatcher::SortBufs& sb, uint64_t cnt) {
 static void launch_trace_kernel(const RayBatcher* b, const DeviceScene& ds, const float4* d_rays, uint32_t cnt, int mode, float* t_o, int* f_o,
                                 uint32_t* fetch, cudaStream_t st) {
     cudaMemsetAsync(fetch, 0, sizeof(uint32_t), st);
-    if (mode == CRT_RAY_CLOSEST) {
-        if (ds.wide) k_trace_batch<0, true><<<b->blocks, 128, 0, st>>>(ds.view(), d_rays, cnt, t_o, f_o, fetch);
-        else k_trace_batch<0, false><<<b->blocks, 128, 0, st>>>(ds.view(), d_rays, cnt, t_o, f_o, fetch);
-    } else {
-        if (ds.wide) k_trace_batch<1, true><<<b->blocks, 128, 0, st>>>(ds.view(), d_rays, cnt, t_o, f_o, fetch);
-        else k_trace_batch<1, false><<<b->blocks, 128, 0, st>>>(ds.view(), d_rays, cnt, t_o, f_o, fetch);
-    }
+    with_layout(ds.wide, [&](auto W) {
+        if (mode == CRT_RAY_CLOSEST) k_trace_batch<0, W.value><<<b->blocks, 128, 0, st>>>(ds.view(), d_rays, cnt, t_o, f_o, fetch);
+        else k_trace_batch<1, W.value><<<b->blocks, 128, 0, st>>>(ds.view(), d_rays, cnt, t_o, f_o, fetch);
+    });
 }
 
 // slot: which of the batcher's two sets of ordering buffers (one per pipeline stream)
@@ -354,13 +309,14 @@ static int launch_trace_batch(RayBatcher* b, const DeviceScene& ds, const float4
         sc[a] = ext > 0.0f ? cells / ext : 0.0f;
     }
     const uint32_t nb = (cnt + 255) / 256;
-    k_ray_keys<<<nb, 256, 0, st>>>(d_rays, cnt, ds.bounds[0], ds.bounds[1], ds.bounds[2], sc[0], sc[1], sc[2], sb.k0, sb.v0);
+    k_ray_keys<<<nb, 256, 0, st>>>(d_rays, cnt, ds.bounds[0], ds.bounds[1], ds.bounds[2], sc[0], sc[1], sc[2], sb.k0.get(), sb.v0.get());
     uint64_t* ks = nullptr;
     uint32_t* perm = nullptr;
-    CRT_CUDA(radix_sort_pairs(sb.k0, sb.k1, sb.v0, sb.v1, cnt, (3 * kRaySortCellBits + 3 + 7) / 8, sb.ghist, sb.scratch, st, &ks, &perm));
-    k_gather_rays<<<nb, 256, 0, st>>>(d_rays, perm, cnt, sb.rays);
-    launch_trace_kernel(b, ds, sb.rays, cnt, kind, sb.t, sb.face, fetch, st);
-    k_scatter_hits<<<nb, 256, 0, st>>>(perm, cnt, sb.t, sb.face, t_o, f_o);
+    CRT_CUDA(radix_sort_pairs(sb.k0.get(), sb.k1.get(), sb.v0.get(), sb.v1.get(), cnt, (3 * kRaySortCellBits + 3 + 7) / 8, sb.ghist.get(),
+                              sb.scratch.get(), st, &ks, &perm));
+    k_gather_rays<<<nb, 256, 0, st>>>(d_rays, perm, cnt, sb.rays.get());
+    launch_trace_kernel(b, ds, sb.rays.get(), cnt, kind, sb.t.get(), sb.face.get(), fetch, st);
+    k_scatter_hits<<<nb, 256, 0, st>>>(perm, cnt, sb.t.get(), sb.face.get(), t_o, f_o);
     return CRT_OK;
 }
 
@@ -370,14 +326,14 @@ int trace_rays_device(RayBatcher* b, const DeviceScene& ds, const float4* d_rays
     float ms_total = 0;
     for (uint64_t off = 0; off < n; off += chunk) {
         const uint32_t cnt = (uint32_t)std::min<uint64_t>(chunk, n - off);
-        CRT_CUDA(cudaEventRecord(b->ev_a[0], st));
-        int rc = launch_trace_batch(b, ds, d_rays + 2 * off, cnt, mode, d_t ? d_t + off : nullptr, d_face ? d_face + off : nullptr, b->fetch, st);
+        CRT_CUDA(cudaEventRecord(b->ev_a[0].get(), st));
+        int rc = launch_trace_batch(b, ds, d_rays + 2 * off, cnt, mode, d_t ? d_t + off : nullptr, d_face ? d_face + off : nullptr, b->fetch.get(), st);
         if (rc != CRT_OK) return rc;
         CRT_CUDA(cudaGetLastError());
-        CRT_CUDA(cudaEventRecord(b->ev_b[0], st));
+        CRT_CUDA(cudaEventRecord(b->ev_b[0].get(), st));
         CRT_CUDA(cudaStreamSynchronize(st));
         float ms = 0;
-        CRT_CUDA(cudaEventElapsedTime(&ms, b->ev_a[0], b->ev_b[0]));
+        CRT_CUDA(cudaEventElapsedTime(&ms, b->ev_a[0].get(), b->ev_b[0].get()));
         ms_total += ms;
     }
     if (kernel_ms) *kernel_ms = ms_total;
@@ -418,46 +374,49 @@ int trace_rays_host(RayBatcher* b, const DeviceScene& ds, const float* rays, uin
         uint64_t chunk = env_u32("CRT_BATCH_CHUNK", 4u << 20);
         chunk = std::max<uint64_t>(1024, std::min<uint64_t>(chunk, 1ull << 28));
         for (int k = 0; k < 2; ++k) {
-            CRT_CUDA(cudaMalloc(&b->d_rays[k], sizeof(float4) * 2 * chunk));
-            CRT_CUDA(cudaMalloc(&b->d_t[k], sizeof(float) * chunk));
-            CRT_CUDA(cudaMalloc(&b->d_face[k], sizeof(int) * chunk));
+            CRT_CUDA(b->d_rays[k].alloc(2 * chunk));
+            CRT_CUDA(b->d_t[k].alloc(chunk));
+            CRT_CUDA(b->d_face[k].alloc(chunk));
         }
         b->chunk = chunk;
     }
     const bool in_place_in = is_page_locked(rays), in_place_t = is_page_locked(t_out), in_place_f = is_page_locked(face_out);
     const uint64_t C = in_place_in && !b->chunk_from_env ? b->chunk / 2 : b->chunk;
     for (int k = 0; k < 2; ++k) {
-        if (!in_place_in && !b->h_rays[k]) CRT_CUDA(cudaHostAlloc((void**)&b->h_rays[k], sizeof(float4) * 2 * b->chunk, cudaHostAllocDefault));
-        if (t_out && !in_place_t && !b->h_t[k]) CRT_CUDA(cudaHostAlloc((void**)&b->h_t[k], sizeof(float) * b->chunk, cudaHostAllocDefault));
-        if (face_out && !in_place_f && !b->h_face[k]) CRT_CUDA(cudaHostAlloc((void**)&b->h_face[k], sizeof(int) * b->chunk, cudaHostAllocDefault));
+        if (!in_place_in && !b->h_rays[k]) CRT_CUDA(pinned_alloc(b->h_rays[k], 2 * b->chunk));
+        if (t_out && !in_place_t && !b->h_t[k]) CRT_CUDA(pinned_alloc(b->h_t[k], b->chunk));
+        if (face_out && !in_place_f && !b->h_face[k]) CRT_CUDA(pinned_alloc(b->h_face[k], b->chunk));
     }
     const uint64_t n_chunks = (n + C - 1) / C;
     float ms_total = 0;
     auto retire = [&](uint64_t k) -> int {                // chunk k has left the GPU: kernel time, staged results to the caller
         const int s = (int)(k & 1);
         const uint64_t off = k * C, cnt = std::min<uint64_t>(C, n - off);
-        CRT_CUDA(cudaEventSynchronize(b->ev_done[s]));
+        CRT_CUDA(cudaEventSynchronize(b->ev_done[s].get()));
         float ms = 0;
-        CRT_CUDA(cudaEventElapsedTime(&ms, b->ev_a[s], b->ev_b[s]));
+        CRT_CUDA(cudaEventElapsedTime(&ms, b->ev_a[s].get(), b->ev_b[s].get()));
         ms_total += ms;
-        if (t_out && !in_place_t) parallel_memcpy(t_out + off, b->h_t[s], sizeof(float) * cnt);
-        if (face_out && !in_place_f) parallel_memcpy(face_out + off, b->h_face[s], sizeof(int) * cnt);
+        if (t_out && !in_place_t) parallel_memcpy(t_out + off, b->h_t[s].get(), sizeof(float) * cnt);
+        if (face_out && !in_place_f) parallel_memcpy(face_out + off, b->h_face[s].get(), sizeof(int) * cnt);
         return CRT_OK;
     };
     for (uint64_t k = 0; k < n_chunks; ++k) {
         const int s = (int)(k & 1);
         const uint64_t off = k * C, cnt = std::min<uint64_t>(C, n - off);
+        cudaStream_t sk = b->st[s].get();
+        float* d_t = b->d_t[s].get();
+        int* d_face = b->d_face[s].get();
         if (k >= 2) { int rc = retire(k - 2); if (rc != CRT_OK) return rc; }      // the slot's buffers are free again
         const float* src = rays + 8 * off;
-        if (!in_place_in) { parallel_memcpy(b->h_rays[s], src, sizeof(float) * 8 * cnt); src = (const float*)b->h_rays[s]; }
-        CRT_CUDA(cudaMemcpyAsync(b->d_rays[s], src, sizeof(float) * 8 * cnt, cudaMemcpyHostToDevice, b->st[s]));
-        CRT_CUDA(cudaEventRecord(b->ev_a[s], b->st[s]));
-        { int rc = launch_trace_batch(b, ds, b->d_rays[s], (uint32_t)cnt, mode, b->d_t[s], b->d_face[s], b->fetch + 32 * s, b->st[s], s); if (rc != CRT_OK) return rc; }
+        if (!in_place_in) { parallel_memcpy(b->h_rays[s].get(), src, sizeof(float) * 8 * cnt); src = (const float*)b->h_rays[s].get(); }
+        CRT_CUDA(cudaMemcpyAsync(b->d_rays[s].get(), src, sizeof(float) * 8 * cnt, cudaMemcpyHostToDevice, sk));
+        CRT_CUDA(cudaEventRecord(b->ev_a[s].get(), sk));
+        { int rc = launch_trace_batch(b, ds, b->d_rays[s].get(), (uint32_t)cnt, mode, d_t, d_face, b->fetch.get() + 32 * s, sk, s); if (rc != CRT_OK) return rc; }
         CRT_CUDA(cudaGetLastError());
-        CRT_CUDA(cudaEventRecord(b->ev_b[s], b->st[s]));
-        if (t_out) CRT_CUDA(cudaMemcpyAsync(in_place_t ? t_out + off : b->h_t[s], b->d_t[s], sizeof(float) * cnt, cudaMemcpyDeviceToHost, b->st[s]));
-        if (face_out) CRT_CUDA(cudaMemcpyAsync(in_place_f ? face_out + off : b->h_face[s], b->d_face[s], sizeof(int) * cnt, cudaMemcpyDeviceToHost, b->st[s]));
-        CRT_CUDA(cudaEventRecord(b->ev_done[s], b->st[s]));
+        CRT_CUDA(cudaEventRecord(b->ev_b[s].get(), sk));
+        if (t_out) CRT_CUDA(cudaMemcpyAsync(in_place_t ? t_out + off : b->h_t[s].get(), d_t, sizeof(float) * cnt, cudaMemcpyDeviceToHost, sk));
+        if (face_out) CRT_CUDA(cudaMemcpyAsync(in_place_f ? face_out + off : b->h_face[s].get(), d_face, sizeof(int) * cnt, cudaMemcpyDeviceToHost, sk));
+        CRT_CUDA(cudaEventRecord(b->ev_done[s].get(), sk));
     }
     for (uint64_t k = n_chunks >= 2 ? n_chunks - 2 : 0; k < n_chunks; ++k) { int rc = retire(k); if (rc != CRT_OK) return rc; }
     if (kernel_ms) *kernel_ms = ms_total;
@@ -558,41 +517,57 @@ struct WfRun {                      // the run_view in flight on a Wavefront (wa
     uint64_t launches = 0;
     unsigned long long w_begin = 0, per_tile32 = 0;       // per_tile32: work items per tile when k_generate takes its 32-bit path, else 0
     float ms_stage[5] = {0, 0, 0, 0, 0};
-    cudaEvent_t se[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    std::vector<std::pair<const char*, cudaEvent_t>> tl;      // CRT_TIMELINE
+    Event se[6];
+    std::vector<std::pair<const char*, Event>> tl;            // CRT_TIMELINE
     void mark(const char* what, cudaStream_t s) {
         if (!timeline) return;
-        cudaEvent_t e;
-        cudaEventCreate(&e);
-        cudaEventRecord(e, s);
-        tl.push_back({what, e});
+        Event e;
+        create(e);
+        cudaEventRecord(e.get(), s);
+        tl.emplace_back(what, std::move(e));
     }
+};
+
+// The path queue of one iteration parity: o (origin, pixel), d (direction, sample), T (throughput, meta), pdf (mis: density of
+// the BSDF sample that produced the ray) and, in scenes with SPECULAR materials, the pending probe rays (o, d, weight) and the
+// list of the paths that have one. The kernels take these as separate __restrict__ pointer parameters: a pointer in a struct
+// parameter, __restrict__ or not, loses the read-only loads (LDG.E.128.CONSTANT) of k_extend, k_shade, k_shadow and k_tail.
+struct PathQueue {
+    DevBuf<float4> o, d, T;
+    DevBuf<float> pdf;
+    DevBuf<float4> pr_o, pr_d, pr_w;
+    DevBuf<uint32_t> pr_list;
+};
+// shadow rays: kShadowRegions regions of region_cap rays; o (origin, tmax), d (direction, pixel), c (contribution)
+struct ShadowQueue {
+    DevBuf<float4> o, d, c;
+    uint32_t region_cap = 0;
+};
+struct PathPool {                  // everything sized by the number of paths in flight
+    uint32_t pool = 0;             // path slots per queue
+    uint32_t shadow_cap = 0;
+    PathQueue q[2];
+    DevBuf<float> hit_t;
+    DevBuf<int> hit_slot, pr_hit;
+    ShadowQueue sh;
 };
 
 struct Wavefront {
     WfRun run;
     uint32_t width = 0, height = 0;
-    uint32_t pool = 0;             // path slots per queue
-    uint32_t shadow_cap = 0, region_cap = 0;      // shadow queue: kShadowRegions regions of region_cap rays
     bool has_probe = false;
-    float4 *q_o[2] = {nullptr, nullptr}, *q_d[2] = {nullptr, nullptr}, *q_T[2] = {nullptr, nullptr};
-    float* q_pdf[2] = {nullptr, nullptr};      // mis: density of the BSDF sample that produced the ray
-    float* hit_t = nullptr;
-    int* hit_slot = nullptr;
-    float4 *pr_o[2] = {nullptr, nullptr}, *pr_d[2] = {nullptr, nullptr}, *pr_w[2] = {nullptr, nullptr};
-    uint32_t* pr_list[2] = {nullptr, nullptr};
-    int* pr_hit = nullptr;
-    float4 *sh_o = nullptr, *sh_d = nullptr, *sh_c = nullptr;
-    long long* accum = nullptr;
-    Counters* counters = nullptr;
-    HostStatus* status_host = nullptr;
+    PathPool paths;
+    DevBuf<long long> accum;
+    DevBuf<Counters> counters;
+    Pinned<HostStatus> status_host;
     HostStatus* status_dev = nullptr;
-    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
-    cudaEvent_t ev_begin = nullptr, ev_end = nullptr;
-    cudaStream_t st_shadow = nullptr;                     // k_shadow of iteration k runs here, beside k_prepare .. k_extend of k + 1
-    cudaEvent_t ev_shaded = nullptr, ev_shadowed = nullptr;
+    Event ev[4];
+    Event ev_begin, ev_end;
+    Stream st_shadow;                                     // k_shadow of iteration k runs here, beside k_prepare .. k_extend of k + 1
+    Event ev_shaded, ev_shadowed;
     int grid_trace = 0, grid_shade = 0, grid_tail = 0;
 };
+void StateDelete::operator()(Wavefront* w) const { delete w; }
 
 // =============================================================================================
 // kernels
@@ -1335,27 +1310,33 @@ int resolve_device(const long long* d_accum, uint32_t n_pixels, uint32_t spp, fl
 // =============================================================================================
 // host driver
 // =============================================================================================
-int wavefront_create(const DeviceScene& ds, uint32_t width, uint32_t height, Wavefront** out) {
-    Wavefront* w = new Wavefront();
-    *out = w;                                        // the caller destroys it when an allocation below fails
+// with_estimator(mis, f): f(integral_constant<int, CRT_ESTIMATOR_MIS or _COMPAT>), for a kernel's EST as E.value
+template <typename F>
+static auto with_estimator(bool mis, F&& f) {
+    return mis ? f(std::integral_constant<int, CRT_ESTIMATOR_MIS>()) : f(std::integral_constant<int, CRT_ESTIMATOR_COMPAT>());
+}
+
+int wavefront_create(const DeviceScene& ds, uint32_t width, uint32_t height, WavefrontPtr& out) {
+    WavefrontPtr w(new Wavefront());
     w->width = width; w->height = height;
     w->has_probe = ds.has_specular;
     const size_t npix = (size_t)width * height;
-    CRT_CUDA(cudaMalloc(&w->accum, sizeof(long long) * 3 * npix));
-    CRT_CUDA(cudaMalloc(&w->counters, sizeof(Counters)));
-    CRT_CUDA(cudaHostAlloc((void**)&w->status_host, sizeof(HostStatus), cudaHostAllocMapped));
-    CRT_CUDA(cudaHostGetDevicePointer((void**)&w->status_dev, (void*)w->status_host, 0));
-    for (int k = 0; k < 4; ++k) CRT_CUDA(cudaEventCreateWithFlags(&w->ev[k], cudaEventDisableTiming));
-    CRT_CUDA(cudaEventCreate(&w->ev_begin));
-    CRT_CUDA(cudaEventCreate(&w->ev_end));
+    CRT_CUDA(w->accum.alloc(3 * npix));
+    CRT_CUDA(w->counters.alloc(1));
+    CRT_CUDA(pinned_alloc(w->status_host, 1, cudaHostAllocMapped));
+    CRT_CUDA(cudaHostGetDevicePointer((void**)&w->status_dev, (void*)w->status_host.get(), 0));
+    for (int k = 0; k < 4; ++k) CRT_CUDA(create(w->ev[k], cudaEventDisableTiming));
+    CRT_CUDA(create(w->ev_begin));
+    CRT_CUDA(create(w->ev_end));
     int occ = 0;
-    if (ds.wide) CRT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_extend<true>, 128, 0));
-    else CRT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_extend<false>, 128, 0));
+    CRT_CUDA(with_layout(ds.wide, [&](auto W) { return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_extend<W.value>, 128, 0); }));
     w->grid_trace = num_sms() * std::max(occ, 1);
     w->grid_shade = num_sms() * 8;
-    if (ds.wide) CRT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, (k_tail<CRT_ESTIMATOR_MIS, true>), 128, 0));
-    else CRT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, (k_tail<CRT_ESTIMATOR_MIS, false>), 128, 0));
+    CRT_CUDA(with_layout(ds.wide, [&](auto W) {
+        return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_tail<CRT_ESTIMATOR_MIS, W.value>, 128, 0);
+    }));
     w->grid_tail = num_sms() * std::max(occ, 1);
+    out = std::move(w);
     return CRT_OK;
 }
 
@@ -1378,61 +1359,35 @@ static int ensure_pool(Wavefront* w, const DeviceScene& ds, const RenderSettings
     const uint64_t region_cap = std::min<uint64_t>(region_paths, pool) * per_vertex;
     uint64_t shadow_cap = region_cap * kShadowRegions;
     if (shadow_cap > 0xffffffffull) { set_error("light_sample_n x lights too large"); return CRT_ERR_INVALID; }
-    if (w->pool == pool && w->shadow_cap >= shadow_cap) return CRT_OK;
-    w->pool = 0;                                     // nothing is valid until every allocation below has succeeded
-    w->shadow_cap = 0;
-    for (int b = 0; b < 2; ++b) {
-        cudaFree(w->q_o[b]); cudaFree(w->q_d[b]); cudaFree(w->q_T[b]); cudaFree(w->q_pdf[b]);
-        cudaFree(w->pr_o[b]); cudaFree(w->pr_d[b]); cudaFree(w->pr_w[b]); cudaFree(w->pr_list[b]);
-        w->q_o[b] = w->q_d[b] = w->q_T[b] = w->pr_o[b] = w->pr_d[b] = w->pr_w[b] = nullptr;
-        w->pr_list[b] = nullptr; w->q_pdf[b] = nullptr;
-    }
-    cudaFree(w->hit_t); cudaFree(w->hit_slot); cudaFree(w->pr_hit); cudaFree(w->sh_o); cudaFree(w->sh_d); cudaFree(w->sh_c);
-    w->hit_t = nullptr; w->hit_slot = nullptr; w->pr_hit = nullptr; w->sh_o = w->sh_d = w->sh_c = nullptr;
-    for (int b = 0; b < 2; ++b) {
-        CRT_CUDA(cudaMalloc(&w->q_o[b], sizeof(float4) * pool));
-        CRT_CUDA(cudaMalloc(&w->q_d[b], sizeof(float4) * pool));
-        CRT_CUDA(cudaMalloc(&w->q_T[b], sizeof(float4) * pool));
-        CRT_CUDA(cudaMalloc(&w->q_pdf[b], sizeof(float) * pool));
+    if (w->paths.pool == pool && w->paths.shadow_cap >= shadow_cap) return CRT_OK;
+    w->paths = PathPool();                           // pool 0: nothing is valid until every allocation below has succeeded
+    PathPool np;
+    for (PathQueue& q : np.q) {
+        CRT_CUDA(q.o.alloc(pool));
+        CRT_CUDA(q.d.alloc(pool));
+        CRT_CUDA(q.T.alloc(pool));
+        CRT_CUDA(q.pdf.alloc(pool));
         if (w->has_probe) {
-            CRT_CUDA(cudaMalloc(&w->pr_o[b], sizeof(float4) * pool));
-            CRT_CUDA(cudaMalloc(&w->pr_d[b], sizeof(float4) * pool));
-            CRT_CUDA(cudaMalloc(&w->pr_w[b], sizeof(float4) * pool));
-            CRT_CUDA(cudaMalloc(&w->pr_list[b], sizeof(uint32_t) * pool));
+            CRT_CUDA(q.pr_o.alloc(pool));
+            CRT_CUDA(q.pr_d.alloc(pool));
+            CRT_CUDA(q.pr_w.alloc(pool));
+            CRT_CUDA(q.pr_list.alloc(pool));
         }
     }
-    CRT_CUDA(cudaMalloc(&w->hit_t, sizeof(float) * pool));
-    CRT_CUDA(cudaMalloc(&w->hit_slot, sizeof(int) * pool));
-    if (w->has_probe) CRT_CUDA(cudaMalloc(&w->pr_hit, sizeof(int) * pool));
-    CRT_CUDA(cudaMalloc(&w->sh_o, sizeof(float4) * shadow_cap));
-    CRT_CUDA(cudaMalloc(&w->sh_d, sizeof(float4) * shadow_cap));
-    CRT_CUDA(cudaMalloc(&w->sh_c, sizeof(float4) * shadow_cap));
-    w->pool = pool;
-    w->shadow_cap = (uint32_t)shadow_cap;
-    w->region_cap = (uint32_t)region_cap;
+    CRT_CUDA(np.hit_t.alloc(pool));
+    CRT_CUDA(np.hit_slot.alloc(pool));
+    if (w->has_probe) CRT_CUDA(np.pr_hit.alloc(pool));
+    CRT_CUDA(np.sh.o.alloc(shadow_cap));
+    CRT_CUDA(np.sh.d.alloc(shadow_cap));
+    CRT_CUDA(np.sh.c.alloc(shadow_cap));
+    np.sh.region_cap = (uint32_t)region_cap;
+    np.pool = pool;
+    np.shadow_cap = (uint32_t)shadow_cap;
+    w->paths = std::move(np);
     return CRT_OK;
 }
 
-void wavefront_destroy(Wavefront* w) {
-    if (!w) return;
-    for (int b = 0; b < 2; ++b) {
-        cudaFree(w->q_o[b]); cudaFree(w->q_d[b]); cudaFree(w->q_T[b]); cudaFree(w->q_pdf[b]);
-        cudaFree(w->pr_o[b]); cudaFree(w->pr_d[b]); cudaFree(w->pr_w[b]); cudaFree(w->pr_list[b]);
-    }
-    cudaFree(w->hit_t); cudaFree(w->hit_slot); cudaFree(w->pr_hit);
-    cudaFree(w->sh_o); cudaFree(w->sh_d); cudaFree(w->sh_c);
-    cudaFree(w->accum); cudaFree(w->counters);
-    if (w->status_host) cudaFreeHost((void*)w->status_host);
-    for (int k = 0; k < 4; ++k) if (w->ev[k]) cudaEventDestroy(w->ev[k]);
-    if (w->ev_begin) cudaEventDestroy(w->ev_begin);
-    if (w->ev_end) cudaEventDestroy(w->ev_end);
-    if (w->ev_shaded) cudaEventDestroy(w->ev_shaded);
-    if (w->ev_shadowed) cudaEventDestroy(w->ev_shadowed);
-    if (w->st_shadow) cudaStreamDestroy(w->st_shadow);
-    delete w;
-}
-
-long long* wavefront_accum(Wavefront* w) { return w->accum; }
+long long* wavefront_accum(Wavefront* w) { return w->accum.get(); }
 
 // A run_view is a small state machine - begin (reset + first settings), step (the host side of ONE wavefront iteration,
 // optionally without blocking), finish (drain + statistics) - so that one host thread can drive the renders of several
@@ -1469,7 +1424,7 @@ int wavefront_begin(Wavefront* w, const DeviceScene& ds, const RenderSettings& r
     }
     {
         const unsigned long long per_tile = (unsigned long long)p.tile_px * p.tile_S;
-        p.tile_fast = (per_tile >= w->pool && per_tile < (1ull << 31)) ? 1u : 0u;
+        p.tile_fast = (per_tile >= w->paths.pool && per_tile < (1ull << 31)) ? 1u : 0u;
         r.per_tile32 = p.tile_fast ? per_tile : 0ull;
     }
     Counters h;
@@ -1478,9 +1433,9 @@ int wavefront_begin(Wavefront* w, const DeviceScene& ds, const RenderSettings& r
     h.work_end = std::max(w_end, w_begin);
     w->status_host->done = 0;
     w->status_host->n_cur = 0;
-    CRT_CUDA(cudaEventRecord(w->ev_begin, st));
-    if (!rs.accumulate) CRT_CUDA(cudaMemsetAsync(w->accum, 0, sizeof(long long) * 3 * npix, st));
-    CRT_CUDA(cudaMemcpyAsync(w->counters, &h, sizeof(h), cudaMemcpyHostToDevice, st));
+    CRT_CUDA(cudaEventRecord(w->ev_begin.get(), st));
+    if (!rs.accumulate) CRT_CUDA(cudaMemsetAsync(w->accum.get(), 0, sizeof(long long) * 3 * npix, st));
+    CRT_CUDA(cudaMemcpyAsync(w->counters.get(), &h, sizeof(h), cudaMemcpyHostToDevice, st));
     r.ds = &ds; r.rs = rs; r.st = st; r.mis = mis; r.w_begin = w_begin;
     r.sv = ds.view();
     r.wide = ds.wide;
@@ -1490,15 +1445,15 @@ int wavefront_begin(Wavefront* w, const DeviceScene& ds, const RenderSettings& r
     // the tail path tracer reserves stash room for every ray a vertex can push; a scene whose vertices push more than half the
     // stash (lights x light_sample_n + 1) finishes with wavefront iterations instead
     if ((uint64_t)std::max<uint32_t>(ds.n_lights, 1) * rs.light_sample_n + 1 > (uint64_t)kTermCap / 2) r.tail_max = 0;
-    if (rs.stage_timing) for (auto& e : r.se) cudaEventCreate(&e);
+    if (rs.stage_timing) for (Event& e : r.se) create(e);
     // CRT_OVERLAP (default on): k_shadow of iteration k runs on a second stream beside k_prepare, k_generate and k_extend
     // of iteration k + 1 (it only adds to the accumulation buffer; its counters are indexed by iteration parity), so the
     // drain of one persistent kernel is filled by the start of the next. k_shade(k + 1) waits for it (one shadow queue).
     r.overlap = !rs.stage_timing && env_u32("CRT_OVERLAP", 1) != 0 && env_u32("CRT_TIMELINE", 0) == 0;
     if (r.overlap && !w->st_shadow) {
-        CRT_CUDA(cudaStreamCreateWithFlags(&w->st_shadow, cudaStreamNonBlocking));
-        CRT_CUDA(cudaEventCreateWithFlags(&w->ev_shaded, cudaEventDisableTiming));
-        CRT_CUDA(cudaEventCreateWithFlags(&w->ev_shadowed, cudaEventDisableTiming));
+        CRT_CUDA(create(w->st_shadow));
+        CRT_CUDA(create(w->ev_shaded, cudaEventDisableTiming));
+        CRT_CUDA(create(w->ev_shadowed, cudaEventDisableTiming));
     }
     // CRT_TIMELINE=1 (profiling aid): an event behind every launch of the frame, printed to stderr at the end - the
     // real schedule (tail kernel and host polling included), one stream
@@ -1523,79 +1478,84 @@ int wavefront_step(Wavefront* w, bool block, bool* done, bool* progressed) {
     const uint32_t tail_max = r.tail_max, it = r.it;
     uint64_t& launches = r.launches;
     float* ms_stage = r.ms_stage;
-    cudaEvent_t* se = r.se;
+    const Event* se = r.se;
     auto mark = [&](const char* what, cudaStream_t s) { r.mark(what, s); };
     (void)ds;
     *done = false;
     if (progressed) *progressed = false;
     {
         if (it >= 2) {
-            if (block) CRT_CUDA(cudaEventSynchronize(w->ev[(it - 2) & 3]));
+            if (block) CRT_CUDA(cudaEventSynchronize(w->ev[(it - 2) & 3].get()));
             else {
-                cudaError_t q = cudaEventQuery(w->ev[(it - 2) & 3]);
+                cudaError_t q = cudaEventQuery(w->ev[(it - 2) & 3].get());
                 if (q == cudaErrorNotReady) return CRT_OK;
                 if (q != cudaSuccess) return cuda_fail(q, "cudaEventQuery");
             }
             if (w->status_host->done) { *done = true; if (progressed) *progressed = true; return CRT_OK; }
         }
         const int cur = it & 1, nxt = cur ^ 1;
-        k_prepare<<<1, 1, 0, st>>>(w->counters, w->pool, tail_max, w->status_dev, cur, r.per_tile32, r.w_begin);
+        Counters* const counters = w->counters.get();
+        long long* const accum = w->accum.get();
+        const PathPool& pp = w->paths;
+        const PathQueue &qc = pp.q[cur], &qn = pp.q[nxt];
+        const ShadowQueue& sh = pp.sh;
+        k_prepare<<<1, 1, 0, st>>>(counters, pp.pool, tail_max, w->status_dev, cur, r.per_tile32, r.w_begin);
         mark("prepare", st);
         // The tail path tracer goes first: when k_prepare hands the remaining paths to it, the other kernels of this iteration are
         // empty, and it needs nothing from k_shadow of the previous iteration (still running on the second stream), which k_shade
         // below has to wait for. On the shipped frames that shadow launch is 0.2 ms the tail now runs beside.
-#define CRT_TAIL_LAUNCH(EST, W)                                                                                              \
-    k_tail<EST, W><<<w->grid_tail, 128, 0, st>>>(sv, w->counters, p, w->q_o[cur], w->q_d[cur], w->q_T[cur], w->q_pdf[cur], w->pr_d[cur], \
-                                                 w->pr_w[cur], w->accum)
-        if (mis) { if (wide) CRT_TAIL_LAUNCH(CRT_ESTIMATOR_MIS, true); else CRT_TAIL_LAUNCH(CRT_ESTIMATOR_MIS, false); }
-        else { if (wide) CRT_TAIL_LAUNCH(CRT_ESTIMATOR_COMPAT, true); else CRT_TAIL_LAUNCH(CRT_ESTIMATOR_COMPAT, false); }
-#undef CRT_TAIL_LAUNCH
+        with_estimator(mis, [&](auto E) {
+            with_layout(wide, [&](auto W) {
+                k_tail<E.value, W.value><<<w->grid_tail, 128, 0, st>>>(sv, counters, p, qc.o.get(), qc.d.get(), qc.T.get(), qc.pdf.get(),
+                                                                       qc.pr_d.get(), qc.pr_w.get(), accum);
+            });
+        });
         mark("tail", st);
-        if (rs.stage_timing) cudaEventRecord(se[0], st);
-        k_generate<<<w->grid_shade, 256, 0, st>>>(w->counters, p, w->q_o[cur], w->q_d[cur], w->q_T[cur], mis ? w->q_pdf[cur] : nullptr);
+        if (rs.stage_timing) cudaEventRecord(se[0].get(), st);
+        k_generate<<<w->grid_shade, 256, 0, st>>>(counters, p, qc.o.get(), qc.d.get(), qc.T.get(), mis ? qc.pdf.get() : nullptr);
         mark("generate", st);
-        if (rs.stage_timing) cudaEventRecord(se[1], st);
-        if (wide) k_extend<true><<<w->grid_trace, 128, 0, st>>>(sv, w->counters, w->q_o[cur], w->q_d[cur], w->hit_t, w->hit_slot);
-        else k_extend<false><<<w->grid_trace, 128, 0, st>>>(sv, w->counters, w->q_o[cur], w->q_d[cur], w->hit_t, w->hit_slot);
+        if (rs.stage_timing) cudaEventRecord(se[1].get(), st);
+        with_layout(wide, [&](auto W) {
+            k_extend<W.value><<<w->grid_trace, 128, 0, st>>>(sv, counters, qc.o.get(), qc.d.get(), pp.hit_t.get(), pp.hit_slot.get());
+        });
         launches += 3;
         if (w->has_probe && !mis) {
-            if (wide) k_probe<true><<<w->grid_trace, 128, 0, st>>>(sv, w->counters, w->pr_list[cur], w->pr_o[cur], w->pr_d[cur], w->hit_slot, w->pr_hit);
-            else k_probe<false><<<w->grid_trace, 128, 0, st>>>(sv, w->counters, w->pr_list[cur], w->pr_o[cur], w->pr_d[cur], w->hit_slot, w->pr_hit);
+            with_layout(wide, [&](auto W) {
+                k_probe<W.value><<<w->grid_trace, 128, 0, st>>>(sv, counters, qc.pr_list.get(), qc.pr_o.get(), qc.pr_d.get(), pp.hit_slot.get(),
+                                                                pp.pr_hit.get());
+            });
             launches++;
         }
         mark("extend", st);
-        if (rs.stage_timing) cudaEventRecord(se[2], st);
-        if (overlap && it > 0) CRT_CUDA(cudaStreamWaitEvent(st, w->ev_shadowed, 0));      // k_shadow(it - 1) still reads the shadow queue
-        if (mis)
-            k_shade<CRT_ESTIMATOR_MIS><<<w->grid_shade, 128, 0, st>>>(sv, w->counters, p, w->q_o[cur], w->q_d[cur], w->q_T[cur], w->q_pdf[cur],
-                                                                       w->q_pdf[nxt], w->hit_t, w->hit_slot, w->pr_w[cur], w->pr_hit, w->q_o[nxt],
-                                                                       w->q_d[nxt], w->q_T[nxt], w->pr_o[nxt], w->pr_d[nxt], w->pr_w[nxt],
-                                                                       w->pr_list[nxt], w->sh_o, w->sh_d, w->sh_c, w->accum, cur, w->region_cap);
-        else
-            k_shade<CRT_ESTIMATOR_COMPAT><<<w->grid_shade, 128, 0, st>>>(sv, w->counters, p, w->q_o[cur], w->q_d[cur], w->q_T[cur], w->q_pdf[cur],
-                                                                          w->q_pdf[nxt], w->hit_t, w->hit_slot, w->pr_w[cur], w->pr_hit, w->q_o[nxt],
-                                                                          w->q_d[nxt], w->q_T[nxt], w->pr_o[nxt], w->pr_d[nxt], w->pr_w[nxt],
-                                                                          w->pr_list[nxt], w->sh_o, w->sh_d, w->sh_c, w->accum, cur, w->region_cap);
+        if (rs.stage_timing) cudaEventRecord(se[2].get(), st);
+        if (overlap && it > 0) CRT_CUDA(cudaStreamWaitEvent(st, w->ev_shadowed.get(), 0));      // k_shadow(it - 1) still reads the shadow queue
+        with_estimator(mis, [&](auto E) {
+            k_shade<E.value><<<w->grid_shade, 128, 0, st>>>(sv, counters, p, qc.o.get(), qc.d.get(), qc.T.get(), qc.pdf.get(), qn.pdf.get(),
+                                                            pp.hit_t.get(), pp.hit_slot.get(), qc.pr_w.get(), pp.pr_hit.get(), qn.o.get(),
+                                                            qn.d.get(), qn.T.get(), qn.pr_o.get(), qn.pr_d.get(), qn.pr_w.get(), qn.pr_list.get(),
+                                                            sh.o.get(), sh.d.get(), sh.c.get(), accum, cur, sh.region_cap);
+        });
         mark("shade", st);
-        if (rs.stage_timing) cudaEventRecord(se[3], st);
+        if (rs.stage_timing) cudaEventRecord(se[3].get(), st);
         cudaStream_t ss = st;
         if (overlap) {
-            CRT_CUDA(cudaEventRecord(w->ev_shaded, st));
-            CRT_CUDA(cudaStreamWaitEvent(w->st_shadow, w->ev_shaded, 0));
-            ss = w->st_shadow;
+            CRT_CUDA(cudaEventRecord(w->ev_shaded.get(), st));
+            CRT_CUDA(cudaStreamWaitEvent(w->st_shadow.get(), w->ev_shaded.get(), 0));
+            ss = w->st_shadow.get();
         }
-        if (wide) k_shadow<true><<<w->grid_trace, 128, 0, ss>>>(sv, w->counters, w->sh_o, w->sh_d, w->sh_c, w->accum, cur, w->region_cap);
-        else k_shadow<false><<<w->grid_trace, 128, 0, ss>>>(sv, w->counters, w->sh_o, w->sh_d, w->sh_c, w->accum, cur, w->region_cap);
-        if (overlap) CRT_CUDA(cudaEventRecord(w->ev_shadowed, ss));
+        with_layout(wide, [&](auto W) {
+            k_shadow<W.value><<<w->grid_trace, 128, 0, ss>>>(sv, counters, sh.o.get(), sh.d.get(), sh.c.get(), accum, cur, sh.region_cap);
+        });
+        if (overlap) CRT_CUDA(cudaEventRecord(w->ev_shadowed.get(), ss));
         mark("shadow", st);
-        if (rs.stage_timing) cudaEventRecord(se[4], st);
+        if (rs.stage_timing) cudaEventRecord(se[4].get(), st);
         launches += 3;
         if (rs.stage_timing) {
-            cudaEventRecord(se[5], st);
-            cudaEventSynchronize(se[5]);
-            for (int k = 0; k < 5; ++k) { float ms = 0; cudaEventElapsedTime(&ms, se[k], se[k + 1]); ms_stage[k] += ms; }
+            cudaEventRecord(se[5].get(), st);
+            cudaEventSynchronize(se[5].get());
+            for (int k = 0; k < 5; ++k) { float ms = 0; cudaEventElapsedTime(&ms, se[k].get(), se[k + 1].get()); ms_stage[k] += ms; }
         }
-        CRT_CUDA(cudaEventRecord(w->ev[it & 3], st));
+        CRT_CUDA(cudaEventRecord(w->ev[it & 3].get(), st));
         CRT_CUDA(cudaGetLastError());
     }
     r.it = it + 1;
@@ -1605,33 +1565,31 @@ int wavefront_step(Wavefront* w, bool block, bool* done, bool* progressed) {
 
 int wavefront_finish(Wavefront* w, crt_render_stats* stats) {
     WfRun& r = w->run;
-    const RenderSettings& rs = r.rs;
     cudaStream_t st = r.st;
     const bool overlap = r.overlap, timeline = r.timeline;
     const uint32_t it = r.it;
     const unsigned long long w_begin = r.w_begin;
     const uint64_t launches = r.launches;
     float* ms_stage = r.ms_stage;
-    cudaEvent_t* se = r.se;
     auto& tl = r.tl;
     Counters h;
     r.active = false;
-    if (overlap && it > 0) CRT_CUDA(cudaStreamWaitEvent(st, w->ev_shadowed, 0));
-    CRT_CUDA(cudaEventRecord(w->ev_end, st));
+    if (overlap && it > 0) CRT_CUDA(cudaStreamWaitEvent(st, w->ev_shadowed.get(), 0));
+    CRT_CUDA(cudaEventRecord(w->ev_end.get(), st));
     CRT_CUDA(cudaStreamSynchronize(st));
-    if (rs.stage_timing) for (int k = 0; k < 6; ++k) cudaEventDestroy(se[k]);
+    for (Event& e : r.se) e.reset();
     if (timeline) {
         float t0 = 0;
         for (size_t k = 1; k < tl.size(); ++k) {
             float ms = 0, at = 0;
-            cudaEventElapsedTime(&ms, tl[k - 1].second, tl[k].second);
-            cudaEventElapsedTime(&at, tl[0].second, tl[k].second);
+            cudaEventElapsedTime(&ms, tl[k - 1].second.get(), tl[k].second.get());
+            cudaEventElapsedTime(&at, tl[0].second.get(), tl[k].second.get());
             fprintf(stderr, "timeline %8.1f us  +%7.1f us  %s\n", at * 1e3f, ms * 1e3f, tl[k].first);
         }
-        for (auto& e : tl) cudaEventDestroy(e.second);
+        tl.clear();
     }
     if (stats) {
-        CRT_CUDA(cudaMemcpy(&h, w->counters, sizeof(h), cudaMemcpyDeviceToHost));
+        CRT_CUDA(cudaMemcpy(&h, w->counters.get(), sizeof(h), cudaMemcpyDeviceToHost));
         memset(stats, 0, sizeof(*stats));
         stats->samples = h.work_end - w_begin;
         stats->extend_rays = h.stat_extend;
@@ -1641,7 +1599,7 @@ int wavefront_finish(Wavefront* w, crt_render_stats* stats) {
         stats->probe_rays = h.stat_probe;
         stats->iterations = h.iterations;
         stats->kernel_launches = launches;
-        CRT_CUDA(cudaEventElapsedTime(&stats->ms_total, w->ev_begin, w->ev_end));
+        CRT_CUDA(cudaEventElapsedTime(&stats->ms_total, w->ev_begin.get(), w->ev_end.get()));
         stats->ms_generate = ms_stage[0]; stats->ms_extend = ms_stage[1]; stats->ms_shade = ms_stage[2]; stats->ms_shadow = ms_stage[3];
         stats->ms_tail = ms_stage[4];
     }
