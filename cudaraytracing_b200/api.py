@@ -117,6 +117,13 @@ def load_library():
         "crt_render_get_rgb8_device": [vp, vp],
         "crt_render_save_png": [vp, C.c_char_p],
         "crt_render_get_stats": [vp, C.POINTER(_Stats)],
+        "crt_render_set_aov": [vp, i32],
+        "crt_render_get_aov": [vp, vp, vp, vp, vp],
+        "crt_render_get_aov_i64": [vp, vp, C.POINTER(f32)],
+        "crt_render_device_aov": [vp, pp, C.POINTER(f32)],
+        "crt_group_set_aov": [vp, i32],
+        "crt_group_get_aov": [vp, vp, vp, vp, vp],
+        "crt_group_get_aov_i64": [vp, vp, C.POINTER(f32)],
         "crt_render_destroy": [vp],
         "crt_group_create": [vp, u32, u32, vp, u32, pp],
         "crt_group_set_params": [vp, u32, f32, u32, u32, i32],
@@ -413,10 +420,42 @@ class Render:
     def save_frame_buffer(self, path):
         _check(self.L.crt_render_save_png(self.h, path.encode()))
 
+    def set_aov(self, on):
+        """AOV buffers for denoisers (include/crt.h crt_render_set_aov): run_view also accumulates first-hit albedo, normal,
+        depth and coverage over the same samples as the colour."""
+        _check(self.L.crt_render_set_aov(self.h, 1 if on else 0))
+
+    def get_aov(self):
+        """dict of albedo (H,W,3), normal (H,W,3), depth (H,W; +inf where no sample hit), coverage (H,W), top row first."""
+        return _aov_images(self.L.crt_render_get_aov, self.h, self.width, self.height)
+
+    def get_aov_i64(self):
+        """(raw int64[W*H*8] fixed-point AOV buffer, depth_unit)"""
+        return _aov_i64(self.L.crt_render_get_aov_i64, self.h, self.width, self.height)
+
+    def device_aov_ptr(self):
+        p = C.c_void_p()
+        _check(self.L.crt_render_device_aov(self.h, C.byref(p), None))
+        return p.value
+
     def stats(self):
         s = _Stats()
         _check(self.L.crt_render_get_stats(self.h, C.byref(s)))
         return {k: getattr(s, k) for k, _ in _Stats._fields_}
+
+
+def _aov_images(fn, h, width, height):
+    d = dict(albedo=np.zeros((height, width, 3), np.float32), normal=np.zeros((height, width, 3), np.float32),
+             depth=np.zeros((height, width), np.float32), coverage=np.zeros((height, width), np.float32))
+    _check(fn(h, _p(d["albedo"]), _p(d["normal"]), _p(d["depth"]), _p(d["coverage"])))
+    return d
+
+
+def _aov_i64(fn, h, width, height):
+    out = np.zeros(width * height * 8, np.int64)
+    unit = C.c_float()
+    _check(fn(h, _p(out), C.byref(unit)))
+    return out, unit.value
 
 
 def _prefer_bundled_nccl():
@@ -475,6 +514,15 @@ class RenderGroup:
 
     def save_frame_buffer(self, path):
         _check(self.L.crt_group_save_png(self.h, os.fsencode(path)))
+
+    def set_aov(self, on):
+        _check(self.L.crt_group_set_aov(self.h, 1 if on else 0))
+
+    def get_aov(self):
+        return _aov_images(self.L.crt_group_get_aov, self.h, self.width, self.height)
+
+    def get_aov_i64(self):
+        return _aov_i64(self.L.crt_group_get_aov_i64, self.h, self.width, self.height)
 
     def stats(self, index=0):
         st, ms = _Stats(), C.c_float()

@@ -28,13 +28,16 @@ struct crt_render {
     bool rendered = false;
     DevBuf<float> d_linear;
     DevBuf<uint8_t> d_rgb8;
+    bool aov_valid = false;             // the AOV buffer covers exactly the samples of the accumulation buffer
+    DevBuf<float> d_aov_out;            // resolved AOVs, allocated by the first crt_render_get_aov
     crt_render_stats stats{};
     // camera of the last run_view (or of the loaded checkpoint): what the accumulation buffer belongs to
     bool cam_set = false;
     float cam_eye[3] = {0, 0, 0}, cam_M[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0}, cam_fovy = 0;
 };
 
-// Checkpoint file: this header, then width*height*3 int64 (little endian).
+// Checkpoint file: this header, then width*height*3 int64 (little endian); when pad is 1 (AOVs on), width*height*8 int64 of the
+// AOV buffer follow, and payload_bytes and payload_fnv1a cover both.
 struct CheckpointHeader {
     char magic[8];
     uint32_t width, height, spp, seed, estimator, light_sample_n;
@@ -42,7 +45,7 @@ struct CheckpointHeader {
     uint32_t scene_hash;          // crt_scene::scene_hash of the scene the buffer was rendered from (0 in files written before round 2)
     uint64_t work_done;
     float eye[3], M[9], fovy;
-    uint32_t pad;
+    uint32_t pad;                 // 1: the payload includes the AOV buffer, 0: colour only (the layout of files written before AOVs)
     uint64_t payload_bytes, payload_fnv1a;
 };
 static const char kCkptMagic[8] = {'C', 'R', 'T', 'C', 'K', 'P', 'T', '1'};
@@ -462,6 +465,7 @@ int crt_render_run_view(crt_render* r, const float eye[3], const float inv_view[
     float tan_half = tanf(fovy_rad / 2);                          // Render.cuh:338, evaluated on the host
     int rc = wavefront_render(r->wf.get(), r->scene->dev, r->rs, eye, inv_view, tan_half, r->stream, &r->stats);
     r->rendered = rc == CRT_OK;
+    r->aov_valid = rc == CRT_OK && r->rs.aov;
     return rc;
     });
 }
@@ -478,6 +482,7 @@ int crt_render_clear_accum(crt_render* r) {
     CHECK_ARG(r, "crt_render_clear_accum: null handle");
     CRT_CUDA(cudaSetDevice(r->scene->dev.device));
     CRT_CUDA(cudaMemsetAsync(wavefront_accum(r->wf.get()), 0, sizeof(int64_t) * 3 * (size_t)r->rs.width * r->rs.height, r->stream));
+    if (long long* aov = wavefront_aov(r->wf.get())) CRT_CUDA(cudaMemsetAsync(aov, 0, sizeof(int64_t) * 8 * (size_t)r->rs.width * r->rs.height, r->stream));
     CRT_CUDA(cudaStreamSynchronize(r->stream));
     r->cam_set = false;
     return CRT_OK;
@@ -489,16 +494,23 @@ int crt_render_save_checkpoint(crt_render* r, const char* path, uint64_t work_do
     CHECK_ARG(r && path, "crt_render_save_checkpoint: null argument");
     CHECK_ARG(work_done <= (uint64_t)r->rs.width * r->rs.height * r->rs.spp, "crt_render_save_checkpoint: work_done exceeds width * height * spp");
     if (!r->cam_set) { set_error("crt_render_save_checkpoint: nothing rendered yet"); return CRT_ERR_STATE; }
+    const bool with_aov = r->rs.aov;
+    if (with_aov && !r->aov_valid) {
+        set_error("crt_render_save_checkpoint: AOVs are on, but the AOV buffer does not cover the accumulation buffer (AOVs were turned on after the last run_view)");
+        return CRT_ERR_STATE;
+    }
     CRT_CUDA(cudaSetDevice(r->scene->dev.device));
-    const size_t n = 3 * (size_t)r->rs.width * r->rs.height;
+    const size_t npix = (size_t)r->rs.width * r->rs.height, n = 3 * npix + (with_aov ? 8 * npix : 0);
     std::vector<int64_t> buf(n);
-    CRT_CUDA(cudaMemcpy(buf.data(), wavefront_accum(r->wf.get()), sizeof(int64_t) * n, cudaMemcpyDeviceToHost));
+    CRT_CUDA(cudaMemcpy(buf.data(), wavefront_accum(r->wf.get()), sizeof(int64_t) * 3 * npix, cudaMemcpyDeviceToHost));
+    if (with_aov) CRT_CUDA(cudaMemcpy(buf.data() + 3 * npix, wavefront_aov(r->wf.get()), sizeof(int64_t) * 8 * npix, cudaMemcpyDeviceToHost));
     CheckpointHeader h;
     memset(&h, 0, sizeof(h));
     memcpy(h.magic, kCkptMagic, 8);
     h.width = r->rs.width; h.height = r->rs.height; h.spp = r->rs.spp; h.seed = r->rs.seed; h.estimator = (uint32_t)r->rs.estimator;
     h.light_sample_n = r->rs.light_sample_n; h.p_rr = r->rs.p_rr; h.work_done = work_done;
     h.scene_hash = r->scene->scene_hash;
+    h.pad = with_aov ? 1u : 0u;
     memcpy(h.eye, r->cam_eye, sizeof(h.eye)); memcpy(h.M, r->cam_M, sizeof(h.M)); h.fovy = r->cam_fovy;
     h.payload_bytes = sizeof(int64_t) * n;
     h.payload_fnv1a = fnv1a64(buf.data(), h.payload_bytes);
@@ -518,7 +530,7 @@ int crt_render_load_checkpoint(crt_render* r, const char* path, uint64_t* work_d
     FILE* f = fopen(path, "rb");
     if (!f) { set_error(std::string("crt_render_load_checkpoint: cannot open ") + path); return CRT_ERR_IO; }
     CheckpointHeader h;
-    const size_t n = 3 * (size_t)r->rs.width * r->rs.height;
+    const size_t npix = (size_t)r->rs.width * r->rs.height, n = 3 * npix + (r->rs.aov ? 8 * npix : 0);
     std::vector<int64_t> buf;
     int rc = CRT_OK;
     if (fread(&h, sizeof(h), 1, f) != 1 || memcmp(h.magic, kCkptMagic, 8) != 0) {
@@ -528,6 +540,10 @@ int crt_render_load_checkpoint(crt_render* r, const char* path, uint64_t* work_d
                memcmp(&h.p_rr, &r->rs.p_rr, sizeof(float)) != 0) {
         set_error("crt_render_load_checkpoint: the checkpoint was written with different render settings "
                   "(width, height, spp, seed, estimator, P_RR, light_sample_n must match)");
+        rc = CRT_ERR_STATE;
+    } else if ((h.pad != 0) != r->rs.aov) {
+        set_error(h.pad ? "crt_render_load_checkpoint: the checkpoint holds AOVs and AOVs are off (crt_render_set_aov(r, 1) first)"
+                        : "crt_render_load_checkpoint: the checkpoint holds no AOVs and AOVs are on (crt_render_set_aov(r, 0) first)");
         rc = CRT_ERR_STATE;
     } else if (h.scene_hash != 0 && h.scene_hash != r->scene->scene_hash) {
         set_error("crt_render_load_checkpoint: the checkpoint was rendered from a different scene");
@@ -546,7 +562,14 @@ int crt_render_load_checkpoint(crt_render* r, const char* path, uint64_t* work_d
     fclose(f);
     if (rc != CRT_OK) return rc;
     CRT_CUDA(cudaSetDevice(r->scene->dev.device));
-    CRT_CUDA(cudaMemcpy(wavefront_accum(r->wf.get()), buf.data(), sizeof(int64_t) * n, cudaMemcpyHostToDevice));
+    CRT_CUDA(cudaMemcpy(wavefront_accum(r->wf.get()), buf.data(), sizeof(int64_t) * 3 * npix, cudaMemcpyHostToDevice));
+    if (r->rs.aov) {
+        rc = wavefront_ensure_aov(r->wf.get(), r->scene->dev.wide, r->stream);
+        if (rc != CRT_OK) return rc;
+        CRT_CUDA(cudaStreamSynchronize(r->stream));
+        CRT_CUDA(cudaMemcpy(wavefront_aov(r->wf.get()), buf.data() + 3 * npix, sizeof(int64_t) * 8 * npix, cudaMemcpyHostToDevice));
+    }
+    r->aov_valid = r->rs.aov;
     memcpy(r->cam_eye, h.eye, sizeof(h.eye)); memcpy(r->cam_M, h.M, sizeof(h.M)); r->cam_fovy = h.fovy;
     r->cam_set = true;
     r->rs.accumulate = true;
@@ -625,6 +648,70 @@ int crt_render_save_png(crt_render* r, const char* path) {
     return write_png(path, rgb.data(), r->rs.width, r->rs.height);
     });
 }
+// ---- AOVs ------------------------------------------------------------------------------------
+int crt_render_set_aov(crt_render* r, int on) {
+    return guarded("crt_render_set_aov", [&]() -> int {
+    CHECK_ARG(r, "crt_render_set_aov: null handle");
+    if (r->rs.accumulate && r->cam_set) {
+        set_error("crt_render_set_aov: accumulate is on and the accumulation buffer holds work (crt_render_clear_accum first); "
+                  "the AOVs would cover only part of the colour's samples");
+        return CRT_ERR_STATE;
+    }
+    r->rs.aov = on != 0;
+    return CRT_OK;
+    });
+}
+
+static int no_aov(const char* fn) {
+    set_error(std::string(fn) + ": no AOVs rendered (turn them on, then run_view)");
+    return CRT_ERR_STATE;
+}
+
+// resolves d_aov (npix pixels) into d_out on the device, then copies the requested images to the host
+static int resolve_aov_to(const long long* d_aov, size_t npix, uint32_t spp, float unit, DevBuf<float>& d_out, cudaStream_t st,
+                          float* albedo, float* normal, float* depth, float* coverage) {
+    if (!d_out.get()) CRT_CUDA(d_out.alloc(8 * npix));
+    int rc = resolve_aov_device(d_aov, (uint32_t)npix, spp, unit, d_out.get(), st);
+    if (rc != CRT_OK) return rc;
+    float* const out[4] = {albedo, normal, depth, coverage};
+    const size_t off[4] = {0, 3 * npix, 6 * npix, 7 * npix}, cnt[4] = {3 * npix, 3 * npix, npix, npix};
+    for (int k = 0; k < 4; ++k)
+        if (out[k]) CRT_CUDA(cudaMemcpyAsync(out[k], d_out.get() + off[k], sizeof(float) * cnt[k], cudaMemcpyDeviceToHost, st));
+    CRT_CUDA(cudaStreamSynchronize(st));
+    return CRT_OK;
+}
+
+int crt_render_get_aov(crt_render* r, float* albedo, float* normal, float* depth, float* coverage) {
+    return guarded("crt_render_get_aov", [&]() -> int {
+    CHECK_ARG(r, "crt_render_get_aov: null handle");
+    if (!r->aov_valid) return no_aov("crt_render_get_aov");
+    CRT_CUDA(cudaSetDevice(r->scene->dev.device));
+    return resolve_aov_to(wavefront_aov(r->wf.get()), (size_t)r->rs.width * r->rs.height, r->rs.spp, aov_depth_unit(r->scene->dev.bounds, r->cam_eye),
+                          r->d_aov_out, r->stream, albedo, normal, depth, coverage);
+    });
+}
+
+int crt_render_get_aov_i64(crt_render* r, int64_t* out, float* depth_unit) {
+    return guarded("crt_render_get_aov_i64", [&]() -> int {
+    CHECK_ARG(r && out, "crt_render_get_aov_i64: null argument");
+    if (!r->aov_valid) return no_aov("crt_render_get_aov_i64");
+    CRT_CUDA(cudaSetDevice(r->scene->dev.device));
+    CRT_CUDA(cudaMemcpy(out, wavefront_aov(r->wf.get()), sizeof(int64_t) * 8 * (size_t)r->rs.width * r->rs.height, cudaMemcpyDeviceToHost));
+    if (depth_unit) *depth_unit = aov_depth_unit(r->scene->dev.bounds, r->cam_eye);
+    return CRT_OK;
+    });
+}
+
+int crt_render_device_aov(crt_render* r, void** d_aov, float* depth_unit) {
+    return guarded("crt_render_device_aov", [&]() -> int {
+    CHECK_ARG(r && d_aov, "crt_render_device_aov: null argument");
+    if (!r->aov_valid) return no_aov("crt_render_device_aov");
+    *d_aov = wavefront_aov(r->wf.get());
+    if (depth_unit) *depth_unit = aov_depth_unit(r->scene->dev.bounds, r->cam_eye);
+    return CRT_OK;
+    });
+}
+
 int crt_render_get_stats(crt_render* r, crt_render_stats* out) {
     return guarded("crt_render_get_stats", [&]() -> int {
     CHECK_ARG(r && out, "crt_render_get_stats: null argument");
@@ -712,6 +799,9 @@ struct crt_group {
     DevBuf<float> d_linear;
     DevBuf<uint8_t> d_rgb8;
     bool rendered = false;
+    bool aov_valid = false;                     // the reduced AOV buffer of the last run_view is on devices[0]
+    float aov_unit = 1.0f;
+    DevBuf<float> d_aov_out;
     const DeviceScene& scene_of(size_t g) const { return g == 0 ? scene->dev : replicas[g]; }
 };
 
@@ -820,6 +910,7 @@ int crt_group_run_view(crt_group* g, const float eye[3], const float inv_view[9]
     const unsigned long long npix = (unsigned long long)g->width * g->height, total = npix * g->rs.spp;
     const float tan_half = tanf(fovy_rad / 2);
     g->rendered = false;
+    g->aov_valid = false;
     // shares of the sample-major work index space: whole samples when spp >= G (every GPU renders whole frames), else pixel ranges
     for (size_t k = 0; k < G; ++k) {
         RenderSettings rs = g->rs;
@@ -877,6 +968,14 @@ int crt_group_run_view(crt_group* g, const float eye[3], const float inv_view[9]
             if (rc != CRT_OK) return rc;
         }
         CRT_CUDA(cudaEventRecord(g->ev_r1.get(), g->streams[0].get()));
+        if (g->rs.aov) {                        // the AOV buffers: one more sum onto devices[0], resolved when they are read
+            CRT_NCCL(g_nccl.GroupStart());
+            for (size_t k = 0; k < G; ++k) {
+                long long* aov = wavefront_aov(g->wf[k].get());
+                CRT_NCCL(g_nccl.Reduce(aov, aov, (size_t)(8 * npix), ncclInt64, ncclSum, 0, g->comms[k], g->streams[k].get()));
+            }
+            CRT_NCCL(g_nccl.GroupEnd());
+        }
         for (size_t k = 0; k < G; ++k) {
             CRT_CUDA(cudaSetDevice(g->devices[k]));
             CRT_CUDA(cudaStreamSynchronize(g->streams[k].get()));
@@ -887,6 +986,8 @@ int crt_group_run_view(crt_group* g, const float eye[3], const float inv_view[9]
         g->resolved = true;
     }
     g->rendered = true;
+    g->aov_valid = g->rs.aov;
+    g->aov_unit = aov_depth_unit(g->scene->dev.bounds, eye);
     return CRT_OK;
     });
 }
@@ -918,6 +1019,35 @@ int crt_group_save_png(crt_group* g, const char* path) {
     int rc = crt_group_get_rgb8(g, rgb.data());
     if (rc != CRT_OK) return rc;
     return write_png(path, rgb.data(), g->width, g->height);
+    });
+}
+
+int crt_group_set_aov(crt_group* g, int on) {
+    return guarded("crt_group_set_aov", [&]() -> int {
+    CHECK_ARG(g, "crt_group_set_aov: null handle");
+    g->rs.aov = on != 0;
+    return CRT_OK;
+    });
+}
+
+int crt_group_get_aov(crt_group* g, float* albedo, float* normal, float* depth, float* coverage) {
+    return guarded("crt_group_get_aov", [&]() -> int {
+    CHECK_ARG(g, "crt_group_get_aov: null handle");
+    if (!g->aov_valid) return no_aov("crt_group_get_aov");
+    CRT_CUDA(cudaSetDevice(g->devices[0]));
+    return resolve_aov_to(wavefront_aov(g->wf[0].get()), (size_t)g->width * g->height, g->rs.spp, g->aov_unit, g->d_aov_out, g->streams[0].get(),
+                          albedo, normal, depth, coverage);
+    });
+}
+
+int crt_group_get_aov_i64(crt_group* g, int64_t* out, float* depth_unit) {
+    return guarded("crt_group_get_aov_i64", [&]() -> int {
+    CHECK_ARG(g && out, "crt_group_get_aov_i64: null argument");
+    if (!g->aov_valid) return no_aov("crt_group_get_aov_i64");
+    CRT_CUDA(cudaSetDevice(g->devices[0]));
+    CRT_CUDA(cudaMemcpy(out, wavefront_aov(g->wf[0].get()), sizeof(int64_t) * 8 * (size_t)g->width * g->height, cudaMemcpyDeviceToHost));
+    if (depth_unit) *depth_unit = g->aov_unit;
+    return CRT_OK;
     });
 }
 

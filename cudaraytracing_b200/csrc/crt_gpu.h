@@ -162,6 +162,7 @@ struct RenderSettings {
     bool range_set = false;
     bool stage_timing = false;
     bool accumulate = false;         // run_view adds to the accumulation buffer instead of clearing it (progressive rendering)
+    bool aov = false;                // run_view also adds the first-hit AOVs of its work range to the AOV buffer
 };
 
 int wavefront_create(const DeviceScene& ds, uint32_t width, uint32_t height, WavefrontPtr& out);
@@ -175,10 +176,19 @@ int wavefront_begin(Wavefront* w, const DeviceScene& ds, const RenderSettings& r
 int wavefront_step(Wavefront* w, bool block, bool* done, bool* progressed);
 int wavefront_finish(Wavefront* w, crt_render_stats* stats);
 long long* wavefront_accum(Wavefront* w);
+// AOV buffer: int64[8 * width * height] (albedo 3, normal 3, depth, coverage; fixed point summed over samples), nullptr until a run
+// with AOVs on, or wavefront_ensure_aov, has allocated it (zeroed, on stream st).
+long long* wavefront_aov(Wavefront* w);
+int wavefront_ensure_aov(Wavefront* w, bool wide, cudaStream_t st);
+// Depth unit of the AOV buffer: the smallest power of two >= the largest distance from the eye to a corner of the scene
+// bounds (in double), 1 when that distance is 0.
+float aov_depth_unit(const float bounds[6], const float eye[3]);
 // Device-to-device replica of a built scene (cudaMemcpyPeer of every table): what the other GPUs of a crt_group get
 // instead of a second parse + build. Leaves `device` selected.
 int clone_scene(const DeviceScene& src, int device, DeviceScene& dst);
 // fixed point -> linear float mean and tone-mapped RGB8 (reference Render.cuh:348,350), on the device
 int resolve_device(const long long* d_accum, uint32_t n_pixels, uint32_t spp, float* d_linear, uint8_t* d_rgb8, cudaStream_t st);
+// AOV buffer -> d_out: albedo[3n], normal[3n], depth[n], coverage[n] (n = n_pixels), on the device
+int resolve_aov_device(const long long* d_aov, uint32_t n_pixels, uint32_t spp, float depth_unit, float* d_out, cudaStream_t st);
 
 }  // namespace crt

@@ -42,6 +42,29 @@ static void resolve(const std::string& obj, const std::string& mtl, const std::s
     *obj_out = obj;
     *mtl_out = mtl;
 }
+// Little-endian PFM (scale -1.0), rows bottom first as the format requires; img is top row first, `channels` 3 (PF) or 1 (Pf).
+static bool write_pfm(const std::string& path, const float* img, uint32_t width, uint32_t height, int channels) {
+    FILE* f = fopen(path.c_str(), "wb");
+    if (!f) return false;
+    bool ok = fprintf(f, "%s\n%u %u\n-1.0\n", channels == 3 ? "PF" : "Pf", width, height) > 0;
+    const size_t row = (size_t)width * channels;
+    for (uint32_t y = height; ok && y-- > 0;) ok = fwrite(img + row * y, sizeof(float), row, f) == row;
+    return (fclose(f) == 0) && ok;
+}
+// --aov PREFIX: PREFIX_albedo.pfm, PREFIX_normal.pfm, PREFIX_depth.pfm of the render (r) or group (g)
+static int write_aov(const std::string& prefix, crt_render* r, crt_group* g, uint32_t width, uint32_t height) {
+    const size_t n = (size_t)width * height;
+    std::vector<float> albedo(3 * n), normal(3 * n), depth(n);
+    const int rc = r ? crt_render_get_aov(r, albedo.data(), normal.data(), depth.data(), nullptr)
+                     : crt_group_get_aov(g, albedo.data(), normal.data(), depth.data(), nullptr);
+    if (rc != CRT_OK) { fprintf(stderr, "crt: get_aov failed: %s\n", crt_last_error()); return 1; }
+    if (!write_pfm(prefix + "_albedo.pfm", albedo.data(), width, height, 3) || !write_pfm(prefix + "_normal.pfm", normal.data(), width, height, 3) ||
+        !write_pfm(prefix + "_depth.pfm", depth.data(), width, height, 1)) {
+        fprintf(stderr, "crt: cannot write %s_*.pfm\n", prefix.c_str());
+        return 1;
+    }
+    return 0;
+}
 static double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
 // The reference's window without the window (src/main.cu:288-378): its widgets as commands read from stdin, the scene and the
@@ -111,7 +134,7 @@ static int run_session(crt_render* render, crt_config cfg) {
 
 int main(int argc, char** argv) {
     std::string config = "config.json", out = "out.png", root = ".";
-    std::string checkpoint;
+    std::string checkpoint, aov;
     bool session = false;
     long spp = -1, seed = -1, width = -1, height = -1, chunk_spp = 64, stop_after = -1;
     int estimator = -1, device = 0, builder = CRT_BUILDER_PLOC8, gpus = 1;
@@ -133,14 +156,17 @@ int main(int argc, char** argv) {
         else if (a == "--chunk-spp") chunk_spp = atol(next());
         else if (a == "--stop-after") stop_after = atol(next());
         else if (a == "--session") session = true;
+        else if (a == "--aov") aov = next();
         else if (a == "--help" || a == "-h") {
             printf("usage: crt --config config.json [--root DIR] [--out image.png] [--spp N] [--seed S]\n"
                    "           [--width W --height H] [--estimator compat|mis] [--builder lbvh|lbvh8|ploc|ploc8] [--device D] [--gpus N]\n"
-                   "           [--checkpoint FILE [--chunk-spp N] [--stop-after CHUNKS]]\n"
+                   "           [--checkpoint FILE [--chunk-spp N] [--stop-after CHUNKS]] [--aov PREFIX]\n"
                    "  --checkpoint: progressive render in chunks of N samples per pixel (default 64); FILE is rewritten after\n"
                    "                every chunk and, if it exists at start, the render resumes from it (bit-identical image).\n"
                    "  --gpus N:     devices D .. D+N-1 render shares of the samples (the built scene is copied device to device), one\n"
                    "                NCCL reduce sums the accumulation buffers on device D; the image is the one a single GPU renders.\n"
+                   "  --aov:        also write first-hit AOVs for a denoiser, over the same samples as the image: PREFIX_albedo.pfm,\n"
+                   "                PREFIX_normal.pfm (3 channels) and PREFIX_depth.pfm (1 channel, +inf where no sample hit).\n"
                    "  --session:    the controls of the reference's window (src/main.cu:288-378) as commands on stdin, the scene staying\n"
                    "                resident between frames: eye X Y Z | lookat X Y Z | up X Y Z | spp N | p_rr P | light_sample_n N |\n"
                    "                render | save [FILE] (default .tmp/<time>.png) | quit. One JSON line per command on stdout.\n");
@@ -183,10 +209,12 @@ int main(int argc, char** argv) {
         double g0 = now_ms();
         DIE_IF(crt_group_create(scene, cfg.width, cfg.height, devs.data(), (uint32_t)devs.size(), &group), "group_create");
         DIE_IF(crt_group_set_params(group, cfg.spp, cfg.p_rr, cfg.light_sample_n, cfg.seed, (int)cfg.estimator), "group_set_params");
+        if (!aov.empty()) DIE_IF(crt_group_set_aov(group, 1), "group_set_aov");
         double g1 = now_ms();
         DIE_IF(crt_group_run_view(group, cfg.eye_pos, M, fovy_rad), "group_run_view");
         double g2 = now_ms();
         DIE_IF(crt_group_save_png(group, out.c_str()), "group_save_png");
+        if (!aov.empty() && write_aov(aov, nullptr, group, cfg.width, cfg.height) != 0) return 1;
         double g3 = now_ms();
         float reduce_ms = 0, slowest = 0;
         unsigned long long ext = 0, sh = 0, pr = 0;
@@ -213,6 +241,10 @@ int main(int argc, char** argv) {
     crt_render_set_light_sample_n(render, cfg.light_sample_n);
     crt_render_set_seed(render, cfg.seed);
     DIE_IF(crt_render_set_estimator(render, (int)cfg.estimator), "set_estimator");
+    if (!aov.empty()) {
+        if (session) { fprintf(stderr, "crt: --aov does not apply to --session\n"); return 2; }
+        DIE_IF(crt_render_set_aov(render, 1), "set_aov");
+    }
     if (session) {
         int rc = run_session(render, cfg);
         crt_render_destroy(render);
@@ -267,6 +299,7 @@ int main(int argc, char** argv) {
     }
     double t4 = now_ms();
     DIE_IF(crt_render_save_png(render, out.c_str()), "save_png");
+    if (!aov.empty() && write_aov(aov, render, nullptr, cfg.width, cfg.height) != 0) return 1;
     double t5 = now_ms();
     double msamples = st.ms_total > 0 ? (double)samples_rendered / (st.ms_total * 1e3) : 0.0;
     printf("{\"triangles\": %llu, \"nodes\": %llu, \"materials\": %u, \"lights\": %u, \"load_ms\": %.2f, \"bvh_build_gpu_ms\": %.3f, "

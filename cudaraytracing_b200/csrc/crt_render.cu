@@ -515,7 +515,8 @@ struct WfRun {                      // the run_view in flight on a Wavefront (wa
     bool wide = false, mis = false, overlap = false, timeline = false;
     uint32_t tail_max = 0, it = 0;
     uint64_t launches = 0;
-    unsigned long long w_begin = 0, per_tile32 = 0;       // per_tile32: work items per tile when k_generate takes its 32-bit path, else 0
+    unsigned long long w_begin = 0, w_end = 0, per_tile32 = 0;
+    float aov_unit = 1.0f;                                  // depth unit of the AOV pass (rs.aov)       // per_tile32: work items per tile when k_generate takes its 32-bit path, else 0
     float ms_stage[5] = {0, 0, 0, 0, 0};
     Event se[6];
     std::vector<std::pair<const char*, Event>> tl;            // CRT_TIMELINE
@@ -558,6 +559,9 @@ struct Wavefront {
     bool has_probe = false;
     PathPool paths;
     DevBuf<long long> accum;
+    DevBuf<long long> aov;                                // 8 per pixel, allocated by the first run with AOVs on
+    DevBuf<uint32_t> aov_fetch;
+    int grid_aov = 0;
     DevBuf<Counters> counters;
     Pinned<HostStatus> status_host;
     HostStatus* status_dev = nullptr;
@@ -610,7 +614,21 @@ __global__ void k_prepare(Counters* c, uint32_t pool, uint32_t tail_max, HostSta
     __threadfence_system();
 }
 
-// Primary rays: reference Render.cuh:338-347 + Ray.cuh:12-15. Work item w -> (sample, pixel) with
+// Direction of the camera ray of (pixel, sample): reference Render.cuh:338-347 + Ray.cuh:12-15. The ray starts at p.eye.
+// k_generate and k_aov both call it, so the AOV pass traces exactly the rays the colour's paths start with.
+CRT_DEV V3 camera_dir(const RenderParamsDev& p, uint32_t pixel, uint32_t sample) {
+    uint32_t i = pixel % p.width, j = pixel / p.width;
+    uint4 r = draw(pixel, sample, kCameraBounce, 0, p.seed);
+    float u1 = u01(r.x), u2 = u01(r.y);
+    float ar = (float)p.width / (float)p.height;
+    float x = (2.0f * ((float)i + u1) / (float)p.width - 1.0f) * p.tan_half * ar;
+    float y = (1.0f - 2.0f * ((float)j + u2) / (float)p.height) * p.tan_half;
+    V3 dc = normalize(mk3(-x, y, 1.0f));
+    V3 d = mk3(dot(mk3(p.M[0], p.M[1], p.M[2]), dc), dot(mk3(p.M[3], p.M[4], p.M[5]), dc), dot(mk3(p.M[6], p.M[7], p.M[8]), dc));
+    return normalize(d);
+}
+
+// Primary rays. Work item w -> (sample, pixel) with
 // consecutive items on consecutive pixels of one sample index (coherent warps, distinct pixels).
 __global__ void __launch_bounds__(256) k_generate(const Counters* __restrict__ c, RenderParamsDev p, float4* __restrict__ q_o,
                                                   float4* __restrict__ q_d, float4* __restrict__ q_T, float* __restrict__ q_pdf) {
@@ -642,15 +660,7 @@ __global__ void __launch_bounds__(256) k_generate(const Counters* __restrict__ c
             pixel = (uint32_t)(w % p.n_pixels);
             sample = p.s_begin + (uint32_t)(w / p.n_pixels);
         }
-        uint32_t i = pixel % p.width, j = pixel / p.width;
-        uint4 r = draw(pixel, sample, kCameraBounce, 0, p.seed);
-        float u1 = u01(r.x), u2 = u01(r.y);
-        float ar = (float)p.width / (float)p.height;
-        float x = (2.0f * ((float)i + u1) / (float)p.width - 1.0f) * p.tan_half * ar;
-        float y = (1.0f - 2.0f * ((float)j + u2) / (float)p.height) * p.tan_half;
-        V3 dc = normalize(mk3(-x, y, 1.0f));
-        V3 d = mk3(dot(mk3(p.M[0], p.M[1], p.M[2]), dc), dot(mk3(p.M[3], p.M[4], p.M[5]), dc), dot(mk3(p.M[6], p.M[7], p.M[8]), dc));
-        d = normalize(d);
+        const V3 d = camera_dir(p, pixel, sample);
         q_o[base + k] = make_float4(p.eye[0], p.eye[1], p.eye[2], __uint_as_float(pixel));
         q_d[base + k] = make_float4(d.x, d.y, d.z, __uint_as_float(sample));
         q_T[base + k] = make_float4(1.0f, 1.0f, 1.0f, __uint_as_float(0u));
@@ -666,6 +676,36 @@ __global__ void __launch_bounds__(128, CRT_MINB) k_extend(SceneView sc, Counters
         sc, c->n_cur, &c->fetch_extend,
         [&](uint32_t i, V3& o, V3& d, float& tmax) { o = mk3(q_o[i]); d = mk3(q_d[i]); tmax = FLT_MAX; return true; },
         [&](uint32_t i, const HitRec& h) { hit_t[i] = h.t; hit_slot[i] = h.slot; });
+}
+
+// AOV pass (DESIGN.md "AOV buffers"): work items [w0, w0 + n) of the run, each the camera ray k_generate makes for it, traced
+// closest-hit; a hit adds albedo (Kd), face normal, depth min(t / depth_unit, 1) and coverage 1 as fixed point to
+// aov[8 * pixel + 0..7]. The AOV parameters are kernel arguments of their own: fields added to RenderParamsDev would move the
+// parameter offsets of every other kernel.
+template <bool WIDE>
+__global__ void __launch_bounds__(128, CRT_MINB) k_aov(SceneView sc, RenderParamsDev p, unsigned long long w0, uint32_t n,
+                                                       long long* __restrict__ aov, float depth_unit, uint32_t* __restrict__ fetch) {
+    trace_queue<0, WIDE>(
+        sc, n, fetch,
+        [&](uint32_t k, V3& o, V3& d, float& tmax) {
+            const unsigned long long w = w0 + k;
+            o = mk3(p.eye[0], p.eye[1], p.eye[2]);
+            d = camera_dir(p, (uint32_t)(w % p.n_pixels), p.s_begin + (uint32_t)(w / p.n_pixels));
+            tmax = FLT_MAX;
+            return true;
+        },
+        [&](uint32_t k, const HitRec& h) {
+            if (h.slot < 0) return;
+            const float4 sh = __ldg(sc.tri_shade + h.slot);
+            const float4 kd = __ldg(sc.mats + 5 * __float_as_uint(sh.w));
+            const float v[8] = {kd.x, kd.y, kd.z, sh.x, sh.y, sh.z, fminf(h.t / depth_unit, 1.0f), 1.0f};
+            unsigned long long* a = (unsigned long long*)(aov + 8 * (size_t)((w0 + k) % p.n_pixels));
+#pragma unroll
+            for (int c = 0; c < 8; ++c) {
+                const long long q = quantize(v[c]);
+                if (q) atomicAdd(a + c, (unsigned long long)q);
+            }
+        });
 }
 
 // SPECULAR probe rays (reference Render.cuh:303): traced only when the continuation ray hit.
@@ -1307,6 +1347,46 @@ int resolve_device(const long long* d_accum, uint32_t n_pixels, uint32_t spp, fl
     return CRT_OK;
 }
 
+// AOV resolve: albedo, normal and coverage are means over spp like k_resolve; depth is the mean over the samples that hit
+// (sum of depths over sum of coverage, in units of depth_unit), +inf where none did.
+__global__ void k_resolve_aov(const long long* __restrict__ aov, uint32_t n_pixels, uint32_t spp, float depth_unit, float* __restrict__ albedo,
+                              float* __restrict__ normal, float* __restrict__ depth, float* __restrict__ coverage) {
+    const uint32_t px = blockIdx.x * blockDim.x + threadIdx.x;
+    if (px >= n_pixels) return;
+    const long long* a = aov + 8 * (size_t)px;
+    for (int c = 0; c < 3; ++c) {
+        albedo[3 * (size_t)px + c] = (float)((double)a[c] / 4294967296.0 / (double)spp);
+        normal[3 * (size_t)px + c] = (float)((double)a[3 + c] / 4294967296.0 / (double)spp);
+    }
+    depth[px] = a[7] == 0 ? __int_as_float(0x7f800000) : (float)((double)a[6] / (double)a[7] * (double)depth_unit);
+    coverage[px] = (float)((double)a[7] / 4294967296.0 / (double)spp);
+}
+
+int resolve_aov_device(const long long* d_aov, uint32_t n_pixels, uint32_t spp, float depth_unit, float* d_out, cudaStream_t st) {
+    const size_t n = n_pixels;
+    k_resolve_aov<<<(n_pixels + 255) / 256, 256, 0, st>>>(d_aov, n_pixels, spp ? spp : 1, depth_unit, d_out, d_out + 3 * n, d_out + 6 * n,
+                                                           d_out + 7 * n);
+    CRT_CUDA(cudaGetLastError());
+    return CRT_OK;
+}
+
+float aov_depth_unit(const float bounds[6], const float eye[3]) {
+    double far2 = 0;
+    for (int c = 0; c < 8; ++c) {
+        double d2 = 0;
+        for (int a = 0; a < 3; ++a) {
+            const double e = (double)bounds[(c >> a & 1) ? 3 + a : a] - (double)eye[a];
+            d2 += e * e;
+        }
+        far2 = std::max(far2, d2);
+    }
+    const double far = sqrt(far2);
+    if (!(far > 0)) return 1.0f;
+    int ex = 0;
+    const double m = frexp(far, &ex);                 // far = m * 2^ex, m in [0.5, 1)
+    return (float)ldexp(1.0, m == 0.5 ? ex - 1 : ex);
+}
+
 // =============================================================================================
 // host driver
 // =============================================================================================
@@ -1388,6 +1468,37 @@ static int ensure_pool(Wavefront* w, const DeviceScene& ds, const RenderSettings
 }
 
 long long* wavefront_accum(Wavefront* w) { return w->accum.get(); }
+long long* wavefront_aov(Wavefront* w) { return w->aov.get(); }
+
+int wavefront_ensure_aov(Wavefront* w, bool wide, cudaStream_t st) {
+    if (w->aov.get()) return CRT_OK;
+    const size_t n = 8 * (size_t)w->width * w->height;
+    int occ = 0;
+    CRT_CUDA(with_layout(wide, [&](auto W) { return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_aov<W.value>, 128, 0); }));
+    CRT_CUDA(w->aov_fetch.alloc(1));
+    CRT_CUDA(w->aov.alloc(n));
+    CRT_CUDA(cudaMemsetAsync(w->aov.get(), 0, sizeof(long long) * n, st));
+    w->grid_aov = num_sms() * std::max(occ, 1);
+    return CRT_OK;
+}
+
+// The AOV pass over the run's work range, on the run's stream behind the wavefront: launches of at most 2^31 work items, because
+// trace_queue counts them in 32 bits.
+static int launch_aov(Wavefront* w) {
+    WfRun& r = w->run;
+    const unsigned long long chunk = 1ull << 31;
+    for (unsigned long long w0 = r.w_begin; w0 < r.w_end; w0 += chunk) {
+        const uint32_t n = (uint32_t)std::min(chunk, r.w_end - w0);
+        CRT_CUDA(cudaMemsetAsync(w->aov_fetch.get(), 0, sizeof(uint32_t), r.st));
+        with_layout(r.wide, [&](auto W) {
+            k_aov<W.value><<<w->grid_aov, 128, 0, r.st>>>(r.sv, r.p, w0, n, w->aov.get(), r.aov_unit, w->aov_fetch.get());
+        });
+        CRT_CUDA(cudaGetLastError());
+        r.launches++;
+    }
+    r.mark("aov", r.st);
+    return CRT_OK;
+}
 
 // A run_view is a small state machine - begin (reset + first settings), step (the host side of ONE wavefront iteration,
 // optionally without blocking), finish (drain + statistics) - so that one host thread can drive the renders of several
@@ -1433,10 +1544,16 @@ int wavefront_begin(Wavefront* w, const DeviceScene& ds, const RenderSettings& r
     h.work_end = std::max(w_end, w_begin);
     w->status_host->done = 0;
     w->status_host->n_cur = 0;
+    if (rs.aov) {
+        rc = wavefront_ensure_aov(w, ds.wide, st);
+        if (rc != CRT_OK) return rc;
+        r.aov_unit = aov_depth_unit(ds.bounds, eye);
+    }
     CRT_CUDA(cudaEventRecord(w->ev_begin.get(), st));
     if (!rs.accumulate) CRT_CUDA(cudaMemsetAsync(w->accum.get(), 0, sizeof(long long) * 3 * npix, st));
+    if (!rs.accumulate && rs.aov) CRT_CUDA(cudaMemsetAsync(w->aov.get(), 0, sizeof(long long) * 8 * npix, st));
     CRT_CUDA(cudaMemcpyAsync(w->counters.get(), &h, sizeof(h), cudaMemcpyHostToDevice, st));
-    r.ds = &ds; r.rs = rs; r.st = st; r.mis = mis; r.w_begin = w_begin;
+    r.ds = &ds; r.rs = rs; r.st = st; r.mis = mis; r.w_begin = w_begin; r.w_end = std::max(w_end, w_begin);
     r.sv = ds.view();
     r.wide = ds.wide;
     r.launches = 0;
@@ -1491,7 +1608,12 @@ int wavefront_step(Wavefront* w, bool block, bool* done, bool* progressed) {
                 if (q == cudaErrorNotReady) return CRT_OK;
                 if (q != cudaSuccess) return cuda_fail(q, "cudaEventQuery");
             }
-            if (w->status_host->done) { *done = true; if (progressed) *progressed = true; return CRT_OK; }
+            if (w->status_host->done) {
+                if (rs.aov) { int rc = launch_aov(w); if (rc != CRT_OK) return rc; }
+                *done = true;
+                if (progressed) *progressed = true;
+                return CRT_OK;
+            }
         }
         const int cur = it & 1, nxt = cur ^ 1;
         Counters* const counters = w->counters.get();

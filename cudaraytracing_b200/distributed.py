@@ -34,6 +34,13 @@ def accum_as_tensor(render, device):
     return torch.as_tensor(DevicePointer(render.device_accum_ptr(), n), device=device)
 
 
+def aov_as_tensor(render, device):
+    """The render's int64 AOV buffer (W*H*8) as a tensor without a copy; after reduce_accum on it, rank 0's get_aov() resolves the sum."""
+    import torch
+    n = render.width * render.height * 8
+    return torch.as_tensor(DevicePointer(render.device_aov_ptr(), n), device=device)
+
+
 def reduce_accum(tensor, dst=0):
     """Sum of the int64 accumulation buffers onto `dst` (one collective)."""
     import torch.distributed as dist

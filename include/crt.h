@@ -210,7 +210,8 @@ int crt_render_clear_accum(crt_render* r);
  * `path` (written to path.tmp, then renamed). load: the file's width, height, spp, seed, estimator, P_RR and
  * light_sample_n must equal the handle's current settings (CRT_ERR_STATE otherwise; CRT_ERR_IO for a truncated or
  * corrupt file - the payload carries an FNV-1a checksum); fills the accumulation buffer, turns accumulate on and
- * returns work_done and the camera (any out pointer may be NULL). A later run_view with a different camera fails with
+ * returns work_done and the camera (any out pointer may be NULL). With AOVs on (crt_render_set_aov) the file also holds the AOV
+ * buffer; load requires the file's AOV flag to equal the handle's setting (CRT_ERR_STATE otherwise). A later run_view with a different camera fails with
  * CRT_ERR_STATE until crt_render_clear_accum is called. */
 int crt_render_save_checkpoint(crt_render* r, const char* path, uint64_t work_done);
 int crt_render_load_checkpoint(crt_render* r, const char* path, uint64_t* work_done, float eye[3], float inv_view[9],
@@ -231,6 +232,24 @@ int crt_render_get_rgb8(crt_render* r, uint8_t* out);
 int crt_render_get_rgb8_device(crt_render* r, void* d_rgb8);
 /* Render::save_frame_buffer, include/Render.cuh:489-493 */
 int crt_render_save_png(crt_render* r, const char* path);
+/* AOV buffers for denoisers (DESIGN.md "AOV buffers"): with on != 0 (default 0), every run_view also traces the camera ray of
+ * each of its work items - the ray the colour's path starts with, same jitter - closest-hit, and adds to aov[8 * pixel + k] the
+ * fixed-point (value * 2^32) albedo (k 0-2: Kd of the hit face's material, columns 0-2 of crt_scene_export_mats), face normal
+ * (3-5, as crt_scene_export_tris returns it, not flipped toward the camera), depth (6: min(t / depth_unit, 1)) and coverage
+ * (7: 1); a miss adds nothing. depth_unit is the smallest power of two >= the largest distance from the eye to a corner of the
+ * scene bounds (1 if that is 0). The buffer is cleared with the accumulation buffer and, like it, bit-identical for any chunking
+ * of the work range and any GPU count. The pass runs after the wavefront, inside ms_total and kernel_launches; with AOVs off
+ * nothing is launched or allocated (the buffer takes 64 bytes per pixel).
+ * set_aov: CRT_ERR_STATE while accumulate is on and the accumulation buffer holds work since the last clear.
+ * get_aov: albedo and normal n*3, depth and coverage n floats (n = width*height, top row first, any pointer may be NULL);
+ * albedo, normal, coverage are the sums / 2^32 / spp, depth the mean over the samples that hit (in scene units), +inf where none did.
+ * get_aov_i64: the raw int64[n*8] buffer and depth_unit. device_aov: its device pointer (for a caller-side int64 sum across GPUs,
+ * as crt_render_device_accum). Every get returns CRT_ERR_STATE until a run_view with AOVs on (or a checkpoint with AOVs) has
+ * filled the buffer for the current accumulation. */
+int crt_render_set_aov(crt_render* r, int on);
+int crt_render_get_aov(crt_render* r, float* albedo, float* normal, float* depth, float* coverage);
+int crt_render_get_aov_i64(crt_render* r, int64_t* out, float* depth_unit);
+int crt_render_device_aov(crt_render* r, void** d_aov, float* depth_unit);
 int crt_render_get_stats(crt_render* r, crt_render_stats* out);
 /* 1: time every wavefront stage with CUDA events (slower; for profiles). Default 0. */
 int crt_render_set_stage_timing(crt_render* r, int on);
@@ -254,6 +273,11 @@ int crt_group_run_view(crt_group* g, const float eye[3], const float inv_view[9]
 int crt_group_get_accum_i64(crt_group* g, int64_t* out);
 int crt_group_get_rgb8(crt_group* g, uint8_t* out);
 int crt_group_save_png(crt_group* g, const char* path);
+/* AOVs for the group (see crt_render_set_aov): each GPU runs the AOV pass over its share, one more ncclReduce sums the int64 AOV
+ * buffers onto devices[0]; raw and resolved AOVs are bit-identical to a single GPU's. */
+int crt_group_set_aov(crt_group* g, int on);
+int crt_group_get_aov(crt_group* g, float* albedo, float* normal, float* depth, float* coverage);
+int crt_group_get_aov_i64(crt_group* g, int64_t* out, float* depth_unit);
 /* Statistics of GPU `index` (0 .. n_devices-1) for the last run_view; reduce_ms (optional) = CUDA-event time of the ncclReduce. */
 int crt_group_get_stats(crt_group* g, uint32_t index, crt_render_stats* out, float* reduce_ms);
 int crt_group_destroy(crt_group* g);
